@@ -5,9 +5,10 @@ Workload (BASELINE.json configs[1]): one synthetic 346x260 event sequence per st
 31,500 events, 5-bin voxels, batch 1, assumed cfg of SURVEY.md section 8, seed-0 random weights,
 fused voxelise + UNet on one B200.  With N GPUs every rank processes its own sequences (weak scaling).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--precision bf16|fp32]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--precision bf16|fp32] [--dump-outputs DIR]
 
-Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
+Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.  Inputs and weights come from fixed seeds,
+so runs with the same arguments compute on identical inputs; --dump-outputs DIR writes the frames of the last timed step.
 """
 import argparse
 import json
@@ -179,7 +180,7 @@ def run_reference_arm(args, rank, world):
         for _ in range(max(0, min(args.warmup, 1))):
             cpu_reference_fps(2)
         times = []
-        for _ in range(max(1, min(args.steps, 3))):
+        for _ in range(args.steps):
             fps, dt, threads, kind = cpu_reference_fps(T_s)
             times.append(dt)
         sample = "%d of %d windows of one 346x260 sequence" % (T_s, args.windows)
@@ -213,6 +214,23 @@ def workload_config(args, T, note=None):
     return c
 
 
+DUMP_BYTES = 60 << 20
+
+
+def dump_outputs(path, seqs):
+    """Write the frames a caller of the timed path received (per sequence, in stream order, its T frames [1, 1, H, W]) so
+    that two builds can be compared output for output.  ``frames.npy`` (float32 [sequences, T, K]) holds every frame at
+    the same K pixels: all of them when the frames fit in DUMP_BYTES, else a sample drawn with seed 0, whose flat
+    indices y * W + x are ``frame_pixels.npy`` (float64)."""
+    os.makedirs(path, exist_ok=True)
+    frames = torch.stack([torch.cat(f, 0) for f in seqs]).flatten(2)
+    n, t, p = frames.shape
+    k = min(p, DUMP_BYTES // (4 * n * t + 8))
+    pix = np.sort(np.random.default_rng(0).permutation(p)[:k])
+    np.save(os.path.join(path, "frames.npy"), frames[:, :, torch.from_numpy(pix).to(frames.device)].float().cpu().numpy())
+    np.save(os.path.join(path, "frame_pixels.npy"), pix.astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------------
 # GPU arm
 # ------------------------------------------------------------------------------------------------
@@ -234,7 +252,13 @@ def main():
     ap.add_argument("--no-kernel-timing", action="store_true")
     ap.add_argument("--concurrent", type=int, default=2, help="CUDA streams (independent model calls in flight) per GPU")
     ap.add_argument("--batch", type=int, default=8, help="independent sequences batched into each model call")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the frames of the last resident step to DIR/*.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "default"):
+        ap.error("--dump-outputs writes the frames of the default GPU workload only")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -304,8 +328,12 @@ def main():
             main.wait_stream(streams[s])
         return res
 
+    last_frames = None
+
     def step_resident(i):
-        return fan_out(lambda s: model.reconstruct_events_batch(pick(resident, i, s), (H, W), slot=s))
+        nonlocal last_frames
+        last_frames = fan_out(lambda s: model.reconstruct_events_batch(pick(resident, i, s), (H, W), slot=s))
+        return last_frames
 
     def step_e2e(i):
         # pinned host arrays go straight into the plan's static device buffers (async H2D on the stream);
@@ -343,6 +371,8 @@ def main():
         sampler.start()
         ms = timed(step_resident, args.steps)
         clocks = sampler.stop()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, [seq for per_stream in last_frames for seq in per_stream])
         for i in range(2):
             step_e2e(i)
         ms_e2e = timed(step_e2e, args.steps)

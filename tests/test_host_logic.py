@@ -167,3 +167,22 @@ def test_bench_contract_without_gpu():
     assert line["cpu_baseline"]["kind"] in ("reference", "port") and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0 and line["value"] > 0
     assert getattr(bench, "VOXEL_BYTES_PER_WINDOW") == 16 * 31500 + 4 * 5 * 260 * 346
+
+
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """--dump-outputs: every frame of every sequence, whole when it fits the byte budget, else at the same seeded pixels."""
+    import numpy as np
+    import bench
+    seqs = [[torch.rand(1, 1, 6, 7) for _ in range(4)] for _ in range(3)]
+    full = torch.stack([torch.cat(s, 0) for s in seqs]).flatten(2).numpy()
+    bench.dump_outputs(str(tmp_path / "all"), seqs)
+    got = np.load(tmp_path / "all" / "frames.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, full)
+    assert np.array_equal(np.load(tmp_path / "all" / "frame_pixels.npy"), np.arange(42))
+    monkeypatch.setattr(bench, "DUMP_BYTES", 10 * (4 * 3 * 4 + 8))
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), seqs)
+    pix = np.load(tmp_path / "a" / "frame_pixels.npy")
+    got = np.load(tmp_path / "a" / "frames.npy")
+    assert pix.dtype == np.float64 and len(set(pix)) == 10 and np.array_equal(pix, np.load(tmp_path / "b" / "frame_pixels.npy"))
+    assert got.shape == (3, 4, 10) and np.array_equal(got, full[:, :, pix.astype(int)])
