@@ -13,13 +13,15 @@ parameter containers; all arithmetic runs in libbde2vid_sm100.so (head / encoder
 conv with the pointwise update in its epilogue, ResidualBlock with the residual + ReLU in the second conv's
 epilogue, bilinear x2 of (skip + x) feeding the decoder conv, fused pred + sigmoid).  No CPU path exists.
 """
+import functools
 import os
 
 import torch
 import torch.nn as nn
 
 from . import ops
-from .engine import VOX_CPAD, _Layer, _fold_norm, _pack_conv
+from .engine import (VOX_CPAD, _Layer, _conv_layer, _f32, _fold_norm, _gru_layers, _lstm_layer, _pack_conv,
+                     _run_layer)
 from .model import _ConvLayer, _RecurrentConv, _unsupported
 from .ops import ACT_NONE, ACT_RELU, ENGINE_SIMT, ENGINE_TCGEN05, EPI_GRU_OUT, EPI_GRU_UR, EPI_LSTM
 from .registry import MODELS
@@ -64,34 +66,6 @@ class GRUState:
     @property
     def h(self):
         return self.h32_nhwc.permute(0, 3, 1, 2).contiguous()
-
-
-def _gru_layers(blk, dt, tc, pad_to=None):
-    """[update | reset] rows interleaved n = 2c + g, and out_gate (engine.Engine uses the same packing).  ``pad_to``
-    zero-pads the hidden / input channel count (FireNet: 16 -> 32, the tcgen05 tiles need N % 32 == 0)."""
-    def grow(w, b):
-        if pad_to is None:
-            return w, b
-        hid, cin2 = w.shape[0], w.shape[1]
-        cin = cin2 // 2
-        wp = torch.zeros(pad_to, 2 * pad_to, *w.shape[2:], device=w.device)
-        wp[:hid, :cin] = w[:, :cin]
-        wp[:hid, pad_to:pad_to + cin] = w[:, cin:]
-        bp = torch.zeros(pad_to, device=w.device)
-        bp[:hid] = b
-        return wp, bp
-    wu, bu = grow(blk.update_gate.weight.detach().float(), blk.update_gate.bias.detach().float())
-    wr, br = grow(blk.reset_gate.weight.detach().float(), blk.reset_gate.bias.detach().float())
-    wo, bo = grow(blk.out_gate.weight.detach().float(), blk.out_gate.bias.detach().float())
-    hid = wu.shape[0]
-    w = torch.stack([wu, wr], 1).reshape(2 * hid, *wu.shape[1:])
-    b = torch.stack([bu, br], 1).reshape(-1)
-    cm = tc and hid % 64 == 0
-    k = wu.shape[-1]
-    pw, ld = _pack_conv(w, dt, chunk_major=cm)
-    ur = _Layer(pw, ld, b.contiguous(), 2 * hid, k, 1, k // 2, k_order=int(cm))
-    po, ldo = _pack_conv(wo, dt, chunk_major=cm)
-    return ur, _Layer(po, ldo, bo.contiguous(), hid, k, 1, k // 2, k_order=int(cm))
 
 
 class UNetRecurrent(nn.Module):
@@ -151,34 +125,16 @@ class UNetRecurrent(nn.Module):
             return self._packed
         tc = self.precision == "bf16"
         dt = torch.bfloat16 if tc else torch.float32
-        f32 = lambda t: t.detach().to(torch.float32).contiguous()  # noqa: E731
-
-        def conv_layer(holder, stride, cin_pad=None):
-            conv = getattr(holder, "conv2d", holder)
-            wf, bf = _fold_norm(conv, holder if conv is not holder else None)   # eval-mode BN / IN folded in
-            k = wf.shape[-1]
-            cm = tc and k > 1 and wf.shape[1] % 64 == 0
-            w, ld = _pack_conv(wf, dt, cin_pad, chunk_major=cm)
-            return _Layer(w, ld, bf.contiguous(), wf.shape[0], k, stride, k // 2, k_order=int(cm))
-
-        def lstm_layer(conv):   # rows reordered to n = 4*c + gate (in, remember, out, cell: e2vid/submodules.py:292)
-            w = conv.weight.detach().float()
-            hid = w.shape[0] // 4
-            w = w.view(4, hid, *w.shape[1:]).permute(1, 0, 2, 3, 4).reshape(4 * hid, *w.shape[1:])
-            b = conv.bias.detach().float().view(4, hid).t().reshape(-1)
-            cm = tc and hid % 64 == 0
-            pw, ld = _pack_conv(w, dt, chunk_major=cm)
-            return _Layer(pw, ld, b.contiguous(), 4 * hid, 3, 1, 1, k_order=int(cm))
-
         with torch.no_grad():
             self._packed = dict(
                 key=key, dtype=dt, engine=ENGINE_TCGEN05 if tc else ENGINE_SIMT,
-                head=conv_layer(self.head, 1, cin_pad=VOX_CPAD),
-                enc=[(conv_layer(e.conv, 2), lstm_layer(e.recurrent_block.Gates) if self.recurrent_block_type == 'convlstm'
-                      else _gru_layers(e.recurrent_block, dt, tc)) for e in self.encoders],
-                res=[(conv_layer(r.conv1, 1), conv_layer(r.conv2, 1)) for r in self.resblocks],
-                dec=[conv_layer(d, 1) for d in self.decoders],
-                pred_w=f32(self.pred.conv2d.weight.reshape(-1)), pred_b=f32(self.pred.conv2d.bias))
+                head=_conv_layer(self.head, 1, dt, tc, cin_pad=VOX_CPAD),
+                enc=[(_conv_layer(e.conv, 2, dt, tc), _lstm_layer(e.recurrent_block.Gates, dt, tc)
+                      if self.recurrent_block_type == 'convlstm' else _gru_layers(e.recurrent_block, dt, tc))
+                     for e in self.encoders],
+                res=[(_conv_layer(r.conv1, 1, dt, tc), _conv_layer(r.conv2, 1, dt, tc)) for r in self.resblocks],
+                dec=[_conv_layer(d, 1, dt, tc) for d in self.decoders],
+                pred_w=_f32(self.pred.conv2d.weight.reshape(-1)), pred_b=_f32(self.pred.conv2d.bias))
             hw, hb = _fold_norm(self.head.conv2d, self.head)
             # dedicated first-layer kernel (planar fp32 voxels -> NHWC bf16): 32 channels, 5x5, as in the BDE2VID engine
             self._packed["head_direct"] = ((hw.contiguous(), hb.contiguous())
@@ -204,11 +160,6 @@ class UNetRecurrent(nn.Module):
         self._bufs = {key: b}
         return b
 
-    def _gemm(self, P, layer, a0, out, n_img, h, w, c0, **kw):
-        return ops.gemm(a0, layer.w, layer.bias, out, n_img=n_img, h_in=h, w_in=w, c0=c0, n=layer.n, ksize=layer.ksize,
-                        stride=layer.stride, pad=layer.pad, w_ld=layer.w_ld, k_order=layer.k_order, engine=P["engine"],
-                        dtype=P["dtype"], **kw)
-
     # ------------------------------------------------------------------------------------
     def forward(self, x, prev_states):
         """x: [N, num_bins, H, W] float32 CUDA; prev_states: None or the ``states`` of the previous call.
@@ -219,6 +170,7 @@ class UNetRecurrent(nn.Module):
             raise RuntimeError("E2VIDRecurrent.forward needs CUDA tensors; no CPU path exists")
         P = self._pack()
         dt = P["dtype"]
+        G = functools.partial(_run_layer, engine=P["engine"], dtype=dt)
         B, bins, H, W = x.shape
         ne, bc = self.num_encoders, self.base_num_channels
         if bins != self.num_bins:
@@ -232,13 +184,13 @@ class UNetRecurrent(nn.Module):
             ops.head_conv(x.to(torch.float32).contiguous(), P["head_direct"][0], P["head_direct"][1], bufs["head"], act=ACT_RELU)
         else:
             ops.pack_voxel_nhwc(x.to(torch.float32).contiguous(), VOX_CPAD, dt, out=bufs["vox8"])
-            self._gemm(P, P["head"], bufs["vox8"], bufs["head"], B, H, W, VOX_CPAD, act=ACT_RELU)
+            G(P["head"], bufs["vox8"], bufs["head"], B, H, W, VOX_CPAD, act=ACT_RELU)
         cur, cc, ch, cw = bufs["head"], bc, H, W
         states = []
         for i in range(ne):
             lv = bufs["lv"][i]
             conv, lstm = P["enc"][i]
-            self._gemm(P, conv, cur, lv["e"], B, ch, cw, cc, act=ACT_RELU)
+            G(conv, cur, lv["e"], B, ch, cw, cc, act=ACT_RELU)
             st = prev_states[i]
             # states are values (the caller may keep them): fresh tensors per step, as in the reference
             h_out = torch.empty(B, lv["h"], lv["w"], lv["C"], dtype=dt, device=x.device)
@@ -247,7 +199,7 @@ class UNetRecurrent(nn.Module):
                 if st is not None and not isinstance(st, LSTMState):      # reference-layout (h, c) NCHW tensors
                     h0, c0 = st
                     st = LSTMState(h0.permute(0, 2, 3, 1).to(dt).contiguous(), c0.permute(0, 2, 3, 1).float().contiguous())
-                self._gemm(P, lstm, lv["e"], h_out, B, lv["h"], lv["w"], lv["C"],
+                G(lstm, lv["e"], h_out, B, lv["h"], lv["w"], lv["C"],
                            a1=lv["zero"] if st is None else st.h_nhwc, c1=lv["C"], epi=EPI_LSTM,
                            c_prev=None if st is None else st.c_nhwc, c_out=c_out)
                 states.append(LSTMState(h_out, c_out))
@@ -260,17 +212,17 @@ class UNetRecurrent(nn.Module):
                 hr = torch.empty_like(h_out)
                 hp = lv["zero"] if st is None else st.h_nhwc
                 hp32 = None if st is None else st.h32_nhwc
-                self._gemm(P, ur, lv["e"], hr, B, lv["h"], lv["w"], lv["C"], a1=hp, c1=lv["C"], epi=EPI_GRU_UR, c_prev=hp32, c_out=u)
-                self._gemm(P, og, lv["e"], h_out, B, lv["h"], lv["w"], lv["C"], a1=hr, c1=lv["C"], epi=EPI_GRU_OUT, c_prev=hp32,
+                G(ur, lv["e"], hr, B, lv["h"], lv["w"], lv["C"], a1=hp, c1=lv["C"], epi=EPI_GRU_UR, c_prev=hp32, c_out=u)
+                G(og, lv["e"], h_out, B, lv["h"], lv["w"], lv["C"], a1=hr, c1=lv["C"], epi=EPI_GRU_OUT, c_prev=hp32,
                            residual=u, c_out=c_out)
                 states.append(GRUState(h_out, c_out))
             cur, cc, ch, cw = h_out, lv["C"], lv["h"], lv["w"]
         # residual blocks: relu(conv2(relu(conv1(x))) + x)   (e2vid/submodules.py:234-247)
         r = bufs["res"]
         for j, (c1l, c2l) in enumerate(P["res"]):
-            self._gemm(P, c1l, cur, r[2], B, ch, cw, cc, act=ACT_RELU)
+            G(c1l, cur, r[2], B, ch, cw, cc, act=ACT_RELU)
             dst = r[j & 1]
-            self._gemm(P, c2l, r[2], dst, B, ch, cw, cc, act=ACT_RELU, residual=cur, res_mode=1)
+            G(c2l, r[2], dst, B, ch, cw, cc, act=ACT_RELU, residual=cur, res_mode=1)
             cur = dst
         # decoders: UpsampleConvLayer(skip_sum(x, block))   (unet.py:193-195; ReLU, e2vid/submodules.py:78-106)
         for i in range(ne):
@@ -278,7 +230,7 @@ class UNetRecurrent(nn.Module):
             dd = bufs["dec"][i]
             blk = states[ne - 1 - i].h_nhwc
             ops.upsample2x_sum(blk, cur, 1.0, B, lv["h"], lv["w"], lv["C"], dd["up"])
-            self._gemm(P, P["dec"][i], dd["up"], dd["out"], B, 2 * lv["h"], 2 * lv["w"], lv["C"], act=ACT_RELU)
+            G(P["dec"][i], dd["up"], dd["out"], B, 2 * lv["h"], 2 * lv["w"], lv["C"], act=ACT_RELU)
             cur = dd["out"]
         ops.pred_sigmoid(cur, bufs["head"], P["pred_w"], P["pred_b"], bc, B * H * W, bufs["img"])
         return bufs["img"].clone().view(B, 1, H, W), states
@@ -395,13 +347,23 @@ class FireNet(nn.Module):
             pw, ld = _pack_conv(wp, dt)
             return _Layer(pw, ld, bp.contiguous(), cout_pad, k, 1, k // 2)
 
+        def pad_gru(w, b):
+            """Zero-pads a gate's hidden and input channels to CP (input = cat[x, h], both halves padded)."""
+            hid, cin = w.shape[0], w.shape[1] // 2
+            wp = torch.zeros(CP, 2 * CP, *w.shape[2:], device=w.device)
+            wp[:hid, :cin] = w[:, :cin]
+            wp[:hid, CP:CP + cin] = w[:, cin:]
+            bp = torch.zeros(CP, device=w.device)
+            bp[:hid] = b
+            return wp, bp
+
         with torch.no_grad():
             pw = torch.zeros(CP, device=dev)
             pw[:self.base_num_channels] = self.pred.conv2d.weight.detach().float().reshape(-1)
             self._packed = dict(
                 key=key, dtype=dt, engine=ENGINE_TCGEN05 if tc else ENGINE_SIMT,
                 head=pad_conv(self.head.conv2d, VOX_CPAD, CP),
-                g=[_gru_layers(self.G1, dt, tc, pad_to=CP), _gru_layers(self.G2, dt, tc, pad_to=CP)],
+                g=[_gru_layers(self.G1, dt, tc, grow=pad_gru), _gru_layers(self.G2, dt, tc, grow=pad_gru)],
                 r=[(pad_conv(self.R1.conv1, CP, CP), pad_conv(self.R1.conv2, CP, CP)),
                    (pad_conv(self.R2.conv1, CP, CP), pad_conv(self.R2.conv2, CP, CP))],
                 pred_w=pw.contiguous(), pred_b=self.pred.conv2d.bias.detach().float().contiguous())
@@ -418,12 +380,10 @@ class FireNet(nn.Module):
         dt, CP = P["dtype"], self.CP
         B, bins, H, W = x.shape
         E = lambda *s, dtype=dt: torch.empty(*s, dtype=dtype, device=x.device)  # noqa: E731
-        G = lambda layer, a0, out, c0, **kw: ops.gemm(a0, layer.w, layer.bias, out, n_img=B, h_in=H, w_in=W, c0=c0, n=layer.n,  # noqa: E731
-                                                      ksize=layer.ksize, stride=1, pad=layer.pad, w_ld=layer.w_ld,
-                                                      engine=P["engine"], dtype=dt, **kw)
+        G = functools.partial(_run_layer, n_img=B, h=H, w=W, engine=P["engine"], dtype=dt)
         vox8 = ops.pack_voxel_nhwc(x.to(torch.float32).contiguous(), VOX_CPAD, dt)
         cur = E(B, H, W, CP)
-        G(P["head"], vox8, cur, VOX_CPAD, act=ACT_RELU)
+        G(P["head"], vox8, cur, c0=VOX_CPAD, act=ACT_RELU)
         zero = torch.zeros(B, H, W, CP, dtype=dt, device=x.device)
         for i in range(2):
             st = self._states[i]
@@ -431,13 +391,13 @@ class FireNet(nn.Module):
             h_out, h32, u, hr = E(B, H, W, CP), E(B, H, W, CP, dtype=torch.float32), E(B, H, W, CP, dtype=torch.float32), E(B, H, W, CP)
             hp = zero if st is None else st.h_nhwc
             hp32 = None if st is None else st.h32_nhwc
-            G(ur, cur, hr, CP, a1=hp, c1=CP, epi=EPI_GRU_UR, c_prev=hp32, c_out=u)
-            G(og, cur, h_out, CP, a1=hr, c1=CP, epi=EPI_GRU_OUT, c_prev=hp32, residual=u, c_out=h32)
+            G(ur, cur, hr, c0=CP, a1=hp, c1=CP, epi=EPI_GRU_UR, c_prev=hp32, c_out=u)
+            G(og, cur, h_out, c0=CP, a1=hr, c1=CP, epi=EPI_GRU_OUT, c_prev=hp32, residual=u, c_out=h32)
             self._states[i] = GRUState(h_out, h32)
             c1l, c2l = P["r"][i]
             y, z = E(B, H, W, CP), E(B, H, W, CP)
-            G(c1l, h_out, y, CP, act=ACT_RELU)
-            G(c2l, y, z, CP, act=ACT_RELU, residual=h_out, res_mode=1)
+            G(c1l, h_out, y, c0=CP, act=ACT_RELU)
+            G(c2l, y, z, c0=CP, act=ACT_RELU, residual=h_out, res_mode=1)
             cur = z
         img = torch.empty(B, H, W, dtype=torch.float32, device=x.device)
         # pred: 1x1 conv, no activation; the kernel computes w . (x + head) so `head` is an all-zero map here

@@ -13,6 +13,7 @@ CUDA graph on its second use so that replay costs one launch from the host.
 Weights are repacked once per engine (K-major [Cout, kh*kw*Cin], gate-interleaved LSTM rows,
 query scale folded into q, relative-position bias pre-gathered).
 """
+import functools
 import os
 import warnings
 from collections import OrderedDict
@@ -103,12 +104,74 @@ def _fold_norm(conv, holder):
     return w * scale.view(-1, 1, 1, 1), b * scale + shift
 
 
+def _f32(t):
+    return t.detach().to(torch.float32).contiguous()
+
+
 class _Layer:
     """Packed weights of one conv / linear."""
 
     def __init__(self, w, w_ld, bias, n, ksize=1, stride=1, pad=0, k_order=0):
         self.w, self.w_ld, self.bias, self.n = w, w_ld, bias, n
         self.ksize, self.stride, self.pad, self.k_order = ksize, stride, pad, k_order
+
+
+def _run_layer(layer, a0, out, n_img, h, w, c0, *, engine, dtype, **kw):
+    """``out`` = ``layer`` applied to the NHWC map ``a0`` [n_img, h, w, c0] by bde_gemm (``kw``: ops.gemm's other options)."""
+    return ops.gemm(a0, layer.w, layer.bias, out, n_img=n_img, h_in=h, w_in=w, c0=c0, n=layer.n, ksize=layer.ksize,
+                    stride=layer.stride, pad=layer.pad, w_ld=layer.w_ld, k_order=layer.k_order, engine=engine, dtype=dtype,
+                    **kw)
+
+
+def _packed_conv(w, b, stride, dt, tc, chunk_ok, cin_pad=None):
+    """Packs conv weights w [Cout, Cin, k, k]: chunk-major K (the L1-friendly im2col order of the tcgen05 convs) where
+    ``chunk_ok`` allows it."""
+    k = w.shape[-1]
+    cm = tc and chunk_ok
+    pw, ld = _pack_conv(w, dt, cin_pad, chunk_major=cm)
+    return _Layer(pw, ld, b.contiguous(), w.shape[0], k, stride, k // 2, k_order=int(cm))
+
+
+def _conv_layer(holder, stride, dt, tc, cin_pad=None):
+    """``holder``: a ConvLayer-like container (conv2d [+ norm_layer], folded in) or a bare nn.Conv2d."""
+    conv = getattr(holder, "conv2d", holder)
+    w, b = _fold_norm(conv, holder if conv is not holder else None)
+    return _packed_conv(w, b, stride, dt, tc, w.shape[-1] > 1 and w.shape[1] % 64 == 0, cin_pad)
+
+
+def _merged_conv_layer(hold_f, hold_b, stride, dt, tc):
+    """forward + backward encoder convs read the same input (...V5.py:129-130): one GEMM with N doubled;
+    output channels [0, C) = forward, [C, 2C) = backward."""
+    wf, bf = _fold_norm(hold_f.conv2d, hold_f)
+    wb, bb = _fold_norm(hold_b.conv2d, hold_b)
+    w = torch.cat([wf, wb], 0)
+    return _packed_conv(w, torch.cat([bf, bb], 0), stride, dt, tc, w.shape[-1] > 1 and w.shape[1] % 64 == 0)
+
+
+def _lstm_layer(conv, dt, tc):
+    """ConvLSTM gates conv with rows reordered so that n = 4*c + gate (gate order in, remember, out, cell:
+    submodules.py:320)."""
+    w = conv.weight.detach().float()
+    hid = w.shape[0] // 4
+    w = w.view(4, hid, *w.shape[1:]).permute(1, 0, 2, 3, 4).reshape(4 * hid, *w.shape[1:])
+    b = conv.bias.detach().float().view(4, hid).t().reshape(-1)
+    return _packed_conv(w, b, 1, dt, tc, hid % 64 == 0)
+
+
+def _gru_layers(blk, dt, tc, grow=None):
+    """ConvGRU (submodules.py:337-375) as two convolutions: [update | reset] with rows interleaved n = 2c + g
+    (BDE_EPI_GRU_UR) and out_gate (BDE_EPI_GRU_OUT).  ``grow`` maps each gate's (weight, bias) before packing."""
+    wb = [(c.weight.detach().float(), c.bias.detach().float()) for c in (blk.update_gate, blk.reset_gate, blk.out_gate)]
+    (wu, bu), (wr, br), (wo, bo) = [grow(w, b) for w, b in wb] if grow is not None else wb
+    hid = wu.shape[0]
+    w = torch.stack([wu, wr], 1).reshape(2 * hid, *wu.shape[1:])
+    b = torch.stack([bu, br], 1).reshape(-1)
+    return _packed_conv(w, b, 1, dt, tc, hid % 64 == 0), _packed_conv(wo, bo, 1, dt, tc, hid % 64 == 0)
+
+
+def _lin_layer(lin, dt, scale=1.0):
+    w, ld = _pack_linear(lin.weight.detach().float(), dt, scale)
+    return _Layer(w, ld, _f32(lin.bias * scale), lin.weight.shape[0])
 
 
 class Engine:
@@ -138,7 +201,7 @@ class Engine:
         self.depths = cfg["depths"]
         self.rec = cfg.get("recurrent_block_type", "convlstm")        # 'convlstm' | 'convgru' | None (useRC=False)
         self.concat = cfg.get("skip_type", "sum") == "concat"
-        self.nwin = cfg.get("nwindow_size")
+        self.nwindow_size = cfg.get("nwindow_size")
         self.net_act = cfg.get("net_act", ACT_RELU)
         self.out_act = cfg.get("out_act", ops.ACT_SIGMOID)
         self.fuse_attn = os.environ.get("BDE2VID_FUSED_ATTN", "1") != "0"
@@ -156,60 +219,10 @@ class Engine:
         if self.bins > VOX_CPAD:
             raise NotImplementedError("num_bins > %d" % VOX_CPAD)
         dt = self.dtype
-        f32 = lambda t: t.detach().to(torch.float32).contiguous()  # noqa: E731
-
         tc = self.gemm_engine == ENGINE_TCGEN05
-
-        def conv_layer(holder, stride, cin_pad=None):
-            """``holder``: a ConvLayer-like container (conv2d [+ norm_layer]) or a bare nn.Conv2d."""
-            conv = getattr(holder, "conv2d", holder)
-            wf, bf = _fold_norm(conv, holder if conv is not holder else None)
-            k = wf.shape[-1]
-            cm = tc and k > 1 and wf.shape[1] % 64 == 0      # chunk-major K: L1-friendly im2col order
-            w, ld = _pack_conv(wf, dt, cin_pad, chunk_major=cm)
-            return _Layer(w, ld, bf.contiguous(), wf.shape[0], k, stride, k // 2, k_order=int(cm))
-
-        def merged_conv_layer(hold_f, hold_b, stride):
-            """forward + backward encoder convs read the same input (...V5.py:129-130): one GEMM with N doubled;
-            output channels [0, C) = forward, [C, 2C) = backward."""
-            wf_, bf_ = _fold_norm(hold_f.conv2d, hold_f)
-            wb_, bb_ = _fold_norm(hold_b.conv2d, hold_b)
-            wcat = torch.cat([wf_, wb_], 0)
-            k = wcat.shape[-1]
-            cm = tc and k > 1 and wcat.shape[1] % 64 == 0
-            w, ld = _pack_conv(wcat, dt, chunk_major=cm)
-            return _Layer(w, ld, torch.cat([bf_, bb_], 0).contiguous(), wcat.shape[0], k, stride, k // 2, k_order=int(cm))
-
-        def gru_layers(blk):
-            """ConvGRU (submodules.py:337-375) as two convolutions: [update | reset] with rows interleaved n = 2c + g
-            (BDE_EPI_GRU_UR) and out_gate (BDE_EPI_GRU_OUT)."""
-            wu, wr = blk.update_gate.weight.detach().float(), blk.reset_gate.weight.detach().float()
-            hid = wu.shape[0]
-            w = torch.stack([wu, wr], 1).reshape(2 * hid, *wu.shape[1:])
-            b = torch.stack([blk.update_gate.bias.detach().float(), blk.reset_gate.bias.detach().float()], 1).reshape(-1)
-            cm = tc and hid % 64 == 0
-            pw, ld = _pack_conv(w, dt, chunk_major=cm)
-            ur = _Layer(pw, ld, b.contiguous(), 2 * hid, 3, 1, 1, k_order=int(cm))
-            po, ldo = _pack_conv(blk.out_gate.weight.detach().float(), dt, chunk_major=cm)
-            o = _Layer(po, ldo, f32(blk.out_gate.bias), hid, 3, 1, 1, k_order=int(cm))
-            return ur, o
-
-        def lstm_layer(conv):
-            # rows reordered so that n = 4*c + gate (gate order in, remember, out, cell: submodules.py:320)
-            w = conv.weight.detach().float()
-            hid = w.shape[0] // 4
-            w = w.view(4, hid, *w.shape[1:]).permute(1, 0, 2, 3, 4).reshape(4 * hid, *w.shape[1:])
-            b = conv.bias.detach().float().view(4, hid).t().reshape(-1)
-            cm = tc and hid % 64 == 0
-            pw, ld = _pack_conv(w, dt, chunk_major=cm)
-            return _Layer(pw, ld, b.contiguous(), 4 * hid, 3, 1, 1, k_order=int(cm))
-
-        def lin_layer(lin, scale=1.0):
-            w, ld = _pack_linear(lin.weight.detach().float(), dt, scale)
-            return _Layer(w, ld, f32(lin.bias * scale), lin.weight.shape[0])
-
+        self.gemm = functools.partial(_run_layer, engine=self.gemm_engine, dtype=dt)
         with torch.no_grad():
-            self.head = conv_layer(gen.head, 1, cin_pad=VOX_CPAD)
+            self.head = _conv_layer(gen.head, 1, dt, tc, cin_pad=VOX_CPAD)
             # dedicated first-layer kernel (planar fp32 voxels -> NHWC bf16, no packing pass): 32 channels, 5x5
             hw, hb_ = _fold_norm(gen.head.conv2d, gen.head)
             self.head_direct = None
@@ -220,14 +233,15 @@ class Engine:
             for l in range(self.L):
                 fe, be = gen.forward_encoder[l], gen.backward_encoder[l]
                 fc, bcv = (fe.conv, be.conv) if self.rec is not None else (fe, be)
-                e = dict(f_conv=conv_layer(fc, 2), b_conv=conv_layer(bcv, 2))
+                e = dict(f_conv=_conv_layer(fc, 2, dt, tc), b_conv=_conv_layer(bcv, 2, dt, tc))
                 if self.rec == "convlstm":
-                    e.update(f_lstm=lstm_layer(fe.recurrent_block.Gates), b_lstm=lstm_layer(be.recurrent_block.Gates))
+                    e.update(f_lstm=_lstm_layer(fe.recurrent_block.Gates, dt, tc),
+                             b_lstm=_lstm_layer(be.recurrent_block.Gates, dt, tc))
                 elif self.rec == "convgru":
-                    e.update(f_gru=gru_layers(fe.recurrent_block), b_gru=gru_layers(be.recurrent_block))
+                    e.update(f_gru=_gru_layers(fe.recurrent_block, dt, tc), b_gru=_gru_layers(be.recurrent_block, dt, tc))
                 # the merged form feeds the chains through pitched TMA descriptors: recurrent encoders only
                 if tc and self.rec is not None and os.environ.get("BDE2VID_MERGE_ENC", "1") != "0":
-                    e["fb_conv"] = merged_conv_layer(fc, bcv, 2)
+                    e["fb_conv"] = _merged_conv_layer(fc, bcv, 2, dt, tc)
                 self.enc.append(e)
             self.attn = []
             n_tok = self.ws[0] * self.ws[1]
@@ -237,21 +251,24 @@ class Engine:
                     C = self.bc * 2 ** (l + 1)
                     hd = C // self.heads
                     # kv tokens per frame: the window's tokens, or nwin0 * nwin1 after the reduction conv (DTransformer.py:172-175)
-                    n_kvf = n_tok if self.nwin is None else self.nwin[0] * self.nwin[1]
+                    n_kvf = n_tok if self.nwindow_size is None else self.nwindow_size[0] * self.nwindow_size[1]
+                    use_mma = (self.nwindow_size is None and dt == torch.bfloat16 and n_tok <= 64 and hd in (4, 8, 16)
+                               and self.heads % 2 == 0 and ops.attention_mma_bias_stride(self.D * n_tok) > 0)
+                    # fused front end (tcgen05 only): LayerNorm folded into the projections.
+                    #   Linear(LN(x)) = (W diag(gamma)) xhat + (W beta + b),  xhat = (x - mean) / sqrt(var + eps)
+                    # q and kv share xhat, so ONE GEMM with N = 3C produces [q | k | v] for every kv token.
+                    # Blocks without it take the unfused route (see attention_routes).
+                    fused = tc and use_mma and C in (64, 128, 256)
                     for blk in gen.feat_attns[l].blocks:
                         a = blk.attn
+                        # weights of every route: proj and fc2 always; the rest only where the block's route can use them
+                        b = dict(proj=_lin_layer(a.proj, dt), fc2=_lin_layer(blk.mlp.fc2, dt), tbl=None)
                         # (DTransformer.py:195-197: only the first N = D * n_kvf columns of the index are used)
                         idx = a.relative_position_index[self.q_ind * n_tok:(self.q_ind + 1) * n_tok, :self.D * n_kvf]
                         bias = a.relative_position_bias_table.detach().float()[idx.reshape(-1)]
                         bias_hmn = bias.reshape(n_tok, self.D * n_kvf, self.heads).permute(2, 0, 1).contiguous()
-                        bias = bias_hmn.permute(0, 2, 1).contiguous()
-                        use_mma = (self.nwin is None and dt == torch.bfloat16 and n_tok <= 64 and hd in (4, 8, 16)
-                                   and self.heads % 2 == 0 and ops.attention_mma_bias_stride(self.D * n_tok) > 0)
-                        # fused front end (tcgen05 only): LayerNorm folded into the projections.
-                        #   Linear(LN(x)) = (W diag(gamma)) xhat + (W beta + b),  xhat = (x - mean) / sqrt(var + eps)
-                        # q and kv share xhat, so ONE GEMM with N = 3C produces [q | k | v] for every kv token.
-                        fused = tc and use_mma and C in (64, 128, 256) and self.nwin is None
-                        qkv_l = fc1_l = kv_l = None
+                        if use_mma:
+                            b["bias_mma"] = ops.pad_bias_for_mma(bias_hmn, self.D * n_tok)
                         if fused:
                             sc = hd ** -0.5
                             Wq, bq = a.q.weight.detach().float(), a.q.bias.detach().float()
@@ -261,50 +278,49 @@ class Engine:
                             Wqkv = torch.cat([sc * Wq * gq[None, :], Wkv * gk[None, :]], 0)
                             bqkv = torch.cat([sc * (Wq @ btq + bq), Wkv @ btk + bkv], 0)
                             w, ld = _pack_linear(Wqkv, dt)
-                            qkv_l = _Layer(w, ld, bqkv.contiguous(), 3 * C)
+                            b["qkv"] = _Layer(w, ld, bqkv.contiguous(), 3 * C)
                             # rows [C, 3C) = k | v: the projection of the neighbour frames, precomputable outside the chain
-                            kv_l = _Layer(w[C:], ld, bqkv[C:].contiguous(), 2 * C)
+                            b["kv_l"] = _Layer(w[C:], ld, bqkv[C:].contiguous(), 2 * C)
                             W1, b1 = blk.mlp.fc1.weight.detach().float(), blk.mlp.fc1.bias.detach().float()
                             g2, bt2 = blk.norm2.weight.detach().float(), blk.norm2.bias.detach().float()
                             w, ld = _pack_linear(W1 * g2[None, :], dt)
-                            fc1_l = _Layer(w, ld, (W1 @ bt2 + b1).contiguous(), 4 * C)
-                        # fully fused attention half (gather + LN + q/k/v + attention [+ proj + scatter]): needs the
-                        # analytic relative-position index so that the bias can be rebuilt from the compact table
-                        tbl = None
-                        if (fused and self.fuse_attn and ops.window_attention_fused_supported(C, self.heads, n_tok, self.D)
-                                and tuple(self.ws) == (7, 7)
-                                and torch.equal(a.relative_position_index.cpu(),
-                                                relative_position_index(self.D, 7, 7))):
-                            rel = 13 * 13
-                            tab = a.relative_position_bias_table.detach().float()
-                            rows = [tab[((self.q_ind - d) + self.D - 1) * rel:((self.q_ind - d) + self.D) * rel] for d in range(self.D)]
-                            tbl = torch.stack(rows, 0).permute(2, 0, 1).contiguous()       # [heads, D, 169]
-                        red = None
-                        if self.nwin is not None:
-                            rc = a.reduction_conv
-                            red = (f32(rc.weight.reshape(rc.weight.shape[0], -1)), f32(rc.bias), n_kvf)
-                        blocks.append(dict(
-                            qkv=qkv_l, kv_l=kv_l, fc1_ln=fc1_l, tbl=tbl, red=red,
-                            bias_mma=ops.pad_bias_for_mma(bias_hmn, self.D * n_tok) if use_mma else None,
-                            nq_g=f32(a.norm_q.weight), nq_b=f32(a.norm_q.bias),
-                            nkv_g=f32(a.norm_kv.weight), nkv_b=f32(a.norm_kv.bias),
-                            q=lin_layer(a.q, hd ** -0.5), kv=lin_layer(a.kv), proj=lin_layer(a.proj),
-                            bias=bias,                              # [heads, D*n_tok, n_tok]
-                            n2_g=f32(blk.norm2.weight), n2_b=f32(blk.norm2.bias),
-                            fc1=lin_layer(blk.mlp.fc1), fc2=lin_layer(blk.mlp.fc2)))
+                            b["fc1_ln"] = _Layer(w, ld, (W1 @ bt2 + b1).contiguous(), 4 * C)
+                            # fully fused attention half (gather + LN + q/k/v + attention [+ proj + scatter]): needs the
+                            # analytic relative-position index so that the bias can be rebuilt from the compact table
+                            if (self.fuse_attn and ops.window_attention_fused_supported(C, self.heads, n_tok, self.D)
+                                    and tuple(self.ws) == (7, 7)
+                                    and torch.equal(a.relative_position_index.cpu(),
+                                                    relative_position_index(self.D, 7, 7))):
+                                rel = 13 * 13
+                                tab = a.relative_position_bias_table.detach().float()
+                                rows = [tab[((self.q_ind - d) + self.D - 1) * rel:((self.q_ind - d) + self.D) * rel]
+                                        for d in range(self.D)]
+                                b["tbl"] = torch.stack(rows, 0).permute(2, 0, 1).contiguous()       # [heads, D, 169]
+                        else:
+                            b.update(nq_g=_f32(a.norm_q.weight), nq_b=_f32(a.norm_q.bias),
+                                     nkv_g=_f32(a.norm_kv.weight), nkv_b=_f32(a.norm_kv.bias),
+                                     q=_lin_layer(a.q, dt, hd ** -0.5), kv=_lin_layer(a.kv, dt),
+                                     n2_g=_f32(blk.norm2.weight), n2_b=_f32(blk.norm2.bias), fc1=_lin_layer(blk.mlp.fc1, dt))
+                            if not use_mma:
+                                b["bias"] = bias_hmn.permute(0, 2, 1).contiguous()       # [heads, D*n_kvf, n_tok]
+                            if self.nwindow_size is not None:
+                                rc = a.reduction_conv
+                                b["red"] = (_f32(rc.weight.reshape(rc.weight.shape[0], -1)), _f32(rc.bias), n_kvf)
+                        blocks.append(b)
                 self.attn.append(blocks)
                 # all blocks' k | v projections stacked: one LayerNorm-GEMM per finished frame (the "past" neighbour)
-                if blocks and all(b["kv_l"] is not None for b in blocks):
+                if blocks and all("kv_l" in b for b in blocks):
                     w_all = torch.cat([b["kv_l"].w for b in blocks], 0).contiguous()
                     b_all = torch.cat([b["kv_l"].bias for b in blocks], 0).contiguous()
                     blocks[0]["kv_all"] = _Layer(w_all, blocks[0]["kv_l"].w_ld, b_all, w_all.shape[0])
             # last level with depth 0: ParseLayer + ResidualBlockNoBN x n (...V5.py:77-80, 261-282)
             self.tail = None
             if self.depths[-1] == 0:
-                self.tail = [(conv_layer(rb.conv1, 1), conv_layer(rb.conv2, 1)) for rb in list(gen.feat_attns[-1])[1:]]
-            self.dec = [conv_layer(gen.decoders[i][1], 1) for i in range(self.L)]
+                self.tail = [(_conv_layer(rb.conv1, 1, dt, tc), _conv_layer(rb.conv2, 1, dt, tc))
+                             for rb in list(gen.feat_attns[-1])[1:]]
+            self.dec = [_conv_layer(gen.decoders[i][1], 1, dt, tc) for i in range(self.L)]
             # skip_type 'concat': 1x1 fusion convolution over cat[skip, x] in front of every decoder (...V5.py:86-93)
-            self.dec_fus = [conv_layer(gen.decoders[i][0], 1) for i in range(self.L)] if self.concat else None
+            self.dec_fus = [_conv_layer(gen.decoders[i][0], 1, dt, tc) for i in range(self.L)] if self.concat else None
             pw, pb = gen.predI[1].weight.detach().float().reshape(-1), gen.predI[1].bias.detach().float()
             if self.concat:
                 # predI = conv1x1(2bc -> bc) then conv1x1(bc -> 1) with nothing in between: one [2bc] vector
@@ -330,11 +346,6 @@ class Engine:
         self.dec_chunk = 8
 
     # ------------------------------------------------------------------------------------
-    def _gemm(self, layer, a0, out, n_img, h, w, c0, **kw):
-        return ops.gemm(a0, layer.w, layer.bias, out, n_img=n_img, h_in=h, w_in=w, c0=c0, n=layer.n,
-                        ksize=layer.ksize, stride=layer.stride, pad=layer.pad, w_ld=layer.w_ld,
-                        k_order=layer.k_order, engine=self.gemm_engine, dtype=self.dtype, **kw)
-
     def plan(self, T, B, Hp, Wp, slot=0):
         """``slot`` selects an independent set of buffers + graph, so that several sequences can be
         in flight at once on different CUDA streams (one slot per stream)."""
@@ -432,6 +443,30 @@ class PairSplit:
         dist.all_reduce(img, op=dist.ReduceOp.SUM, group=self.group)
 
 
+# kernel routes of one attention block (attention_routes; _Plan._attention_block runs them)
+KVPRE = "kvpre"        # window_attention_fused_kvpre: neighbour k | v precomputed once per frame (BDE2VID_ATTN_KVPRE=1)
+WHOLE = "whole"        # window_attention_fused, projection + scatter in the kernel
+SPLIT = "split"        # window_attention_fused to the window output, then the proj + scatter GEMM
+QKV = "qkv"            # LayerNorm-gather qkv GEMM, window_attention_mma_qkv, proj + scatter GEMM
+UNFUSED = "unfused"    # LayerNorm gathers, q and kv GEMMs, attention kernel, proj + scatter, LayerNorm, fc1, fc2
+
+
+def attention_routes(eng, l, C, nwin):
+    """The kernel route of every attention block of level ``l`` (C channels, ``nwin`` windows per frame), and whether
+    the blocks of the fused routes run their MLP as one kernel (else as two GEMMs)."""
+    blocks = eng.attn[l]
+    mlp_fused = eng.fuse_mlp and ops.mlp_fused_supported(C, 4 * C)
+    if (C == 256 and eng.fuse_win256 and eng.kv_pre and nwin >= 64 and list(eng.buf) == [-1, 0, 1] and eng.q_ind == 1
+            and all(b["tbl"] is not None for b in blocks)):
+        return [KVPRE] * len(blocks), mlp_fused
+    # C = 256: the whole-window kernel (gather + LN once per window, projection + scatter fused) once there are enough
+    # windows to fill the SMs with one CTA each; below that (a single sequence has 35 level-3 windows) the per-head-group
+    # kernel's 4 CTAs per window finish sooner
+    whole = C == 64 or (eng.fuse_win256 and nwin >= eng.win256_min)
+    return [(WHOLE if whole else SPLIT) if b["tbl"] is not None else QKV if "qkv" in b else UNFUSED
+            for b in blocks], mlp_fused
+
+
 class _Plan:
     """Static buffers + launch sequence for one (T, B, Hp, Wp)."""
 
@@ -452,7 +487,6 @@ class _Plan:
         self.head = E(N, Hp, Wp, eng.bc)
         self.img = E(N, Hp, Wp, dtype=f32)
         self.lv = []
-        mlp_fused = eng.fuse_mlp
         for l in range(eng.L):
             h, w, C = Hp >> (l + 1), Wp >> (l + 1), eng.bc * 2 ** (l + 1)
             # merged forward / backward encoder conv: the recurrent chains then read channel halves of one [.., 2C] map,
@@ -483,25 +517,24 @@ class _Plan:
                 nwin = tm_plain.shape[0]
                 ntok = ws[0] * ws[1]
                 P = B * h * w
-                blocks = eng.attn[l]
-                d.update(tm=[tm_plain, tm_dil], nwin=nwin, ntok=ntok, xs=E(P, C, dtype=f32), ob=E(nwin * ntok, C))
-                # scratch of the unfused forms, only where a block takes them
-                if any(b["tbl"] is None and b["qkv"] is not None for b in blocks):
+                routes, mlp_fused = attention_routes(eng, l, C, nwin)
+                d.update(tm=[tm_plain, tm_dil], nwin=nwin, ntok=ntok, routes=routes, mlp_fused=mlp_fused,
+                         xs=E(P, C, dtype=f32), ob=E(nwin * ntok, C))
+                # scratch of the routes the blocks take
+                if QKV in routes:
                     d["qkv"] = E(nwin * eng.D * ntok, 3 * C)
-                if any(b["qkv"] is None for b in blocks):
-                    n_kvf = ntok if eng.nwin is None else eng.nwin[0] * eng.nwin[1]
+                if UNFUSED in routes:
+                    n_kvf = ntok if eng.nwindow_size is None else eng.nwindow_size[0] * eng.nwindow_size[1]
                     d.update(qn=E(nwin * ntok, C), kvn=E(nwin * eng.D * n_kvf, C), qb=E(nwin * ntok, C),
                              kvb=E(nwin * eng.D * n_kvf, 2 * C))
-                    if eng.nwin is not None:
+                    if eng.nwindow_size is not None:
                         d["kvr"] = E(nwin * eng.D * n_kvf, C, dtype=f32)
-                if not (mlp_fused and ops.mlp_fused_supported(C, 4 * C) and all(b["fc1_ln"] is not None for b in blocks)):
+                if UNFUSED in routes or not mlp_fused:
                     d.update(yn=E(P, C), hid=E(P, 4 * C))
-                if (C == 256 and eng.fuse_win256 and eng.kv_pre and nwin >= 64 and list(eng.buf) == [-1, 0, 1]
-                        and eng.q_ind == 1 and blocks and "kv_all" in blocks[0]
-                        and all(b["tbl"] is not None for b in blocks)):
+                if KVPRE in routes:
                     # precomputed neighbour k | v: future frames for every block and frame, past frame ping-pong
-                    d["kv_fut"] = E(len(blocks), T, P, 2 * C)
-                    d["kv_past"] = [E(P, len(blocks) * 2 * C) for _ in range(2)]
+                    d["kv_fut"] = E(len(routes), T, P, 2 * C)
+                    d["kv_past"] = [E(P, len(routes) * 2 * C) for _ in range(2)]
                     d["xn_all"] = E(T * P, C)          # LayerNorm'ed (no affine: folded into the weights) features, bf16
                     d["ln_one"] = torch.ones(C, dtype=f32, device=dev)
                     d["ln_zero"] = torch.zeros(C, dtype=f32, device=dev)
@@ -624,15 +657,15 @@ class _Plan:
         first = k == 0
         hprev = d["zero"] if first else hbuf[tprev * B:(tprev + 1) * B]
         if eng.rec == "convlstm":
-            eng._gemm(e[layer_key + "_lstm"], xin, hbuf[t * B:(t + 1) * B], B, h, w, C, a1=hprev, c1=C, epi=EPI_LSTM,
+            eng.gemm(e[layer_key + "_lstm"], xin, hbuf[t * B:(t + 1) * B], B, h, w, C, a1=hprev, c1=C, epi=EPI_LSTM,
                       c_prev=None if first else cbuf[(k + 1) & 1], c_out=cbuf[k & 1], **pitch)
             self.launches += 1
             return
         ur, og = e[layer_key + "_gru"]
         u, hr = (d["ub"], d["hrb"]) if rev else (d["uf"], d["hrf"])
         hm_prev = None if first else cbuf[(k + 1) & 1]
-        eng._gemm(ur, xin, hr, B, h, w, C, a1=hprev, c1=C, epi=EPI_GRU_UR, c_prev=hm_prev, c_out=u, **pitch)
-        eng._gemm(og, xin, hbuf[t * B:(t + 1) * B], B, h, w, C, a1=hr, c1=C, epi=EPI_GRU_OUT, c_prev=hm_prev, residual=u,
+        eng.gemm(ur, xin, hr, B, h, w, C, a1=hprev, c1=C, epi=EPI_GRU_UR, c_prev=hm_prev, c_out=u, **pitch)
+        eng.gemm(og, xin, hbuf[t * B:(t + 1) * B], B, h, w, C, a1=hr, c1=C, epi=EPI_GRU_OUT, c_prev=hm_prev, residual=u,
                   c_out=cbuf[k & 1], **pitch)
         self.launches += 2
 
@@ -662,7 +695,7 @@ class _Plan:
             self.launches += 1
         else:
             ops.pack_voxel_nhwc(self.vox_in.view(N, eng.bins, Hp, Wp), VOX_CPAD, eng.dtype, out=self.vox8)
-            eng._gemm(eng.head, self.vox8, self.head, N, Hp, Wp, VOX_CPAD, act=eng.net_act)
+            eng.gemm(eng.head, self.vox8, self.head, N, Hp, Wp, VOX_CPAD, act=eng.net_act)
             self.launches += 2
         x, xc, xh, xw = self.head, eng.bc, Hp, Wp
         for l in range(eng.L):
@@ -676,7 +709,7 @@ class _Plan:
             if merged:
                 # both directions' encoder convs in one launch over all T (same input, N doubled); each chain then reads
                 # its channel half of the [.., 2C] map through a pitched TMA descriptor
-                eng._gemm(e["fb_conv"], x, d["efb"], N, xh, xw, xc, act=eng.net_act)
+                eng.gemm(e["fb_conv"], x, d["efb"], N, xh, xw, xc, act=eng.net_act)
                 self.launches += 1
             side.wait_stream(main)
             pair = self.pair
@@ -686,7 +719,7 @@ class _Plan:
                 with torch.cuda.stream(main if pair is not None else strm):
                     if not merged:
                         # encoder conv is not recurrent: one launch over all T (...V5.py:129-130, conv part)
-                        eng._gemm(conv, x, src, N, xh, xw, xc, act=eng.net_act)
+                        eng.gemm(conv, x, src, N, xh, xw, xc, act=eng.net_act)
                         self.launches += 1
                     if eng.rec is None:
                         continue                  # useRC=False: the encoder is the ConvLayer alone (...V5.py:255-257)
@@ -738,9 +771,9 @@ class _Plan:
             else:
                 x32, xop = d["tl_zero"], d["tl_zerob"]
             for (c1, c2) in eng.tail:
-                eng._gemm(c1, xop, d["tl_y"], B, h, w, C, act=eng.net_act)
+                eng.gemm(c1, xop, d["tl_y"], B, h, w, C, act=eng.net_act)
                 # conv2 + bias + residual (fp32, after the absent activation): x = x + conv2(.)
-                eng._gemm(c2, d["tl_y"], d["tl_x"], B, h, w, C, out_f32=True, residual=x32,
+                eng.gemm(c2, d["tl_y"], d["tl_x"], B, h, w, C, out_f32=True, residual=x32,
                           out2=d["tl_xb"] if lowp else None)
                 x32, xop = d["tl_x"], d["tl_xb"] if lowp else d["tl_x"]
                 self.launches += 2
@@ -778,7 +811,7 @@ class _Plan:
                 # Quirk Q2: decoder 0 sees cat[feat, feat]
                 skip = self.lv[l_in]["feat_t"][s]
                 xin = skip if i == 0 else cur
-                eng._gemm(eng.dec_fus[i], skip, dd["fus"][:n], n, dd["h"], dd["w"], dd["C"], a1=xin, c1=dd["C"])
+                eng.gemm(eng.dec_fus[i], skip, dd["fus"][:n], n, dd["h"], dd["w"], dd["C"], a1=xin, c1=dd["C"])
                 ops.upsample2x_sum(None, dd["fus"][:n], 1.0, n, dd["h"], dd["w"], dd["C"], dd["up"][:n])
                 self.launches += 1
             else:
@@ -787,7 +820,7 @@ class _Plan:
                     ops.upsample2x_sum(None, feat, 2.0, n, dd["h"], dd["w"], dd["C"], dd["up"][:n])
                 else:
                     ops.upsample2x_sum(feat, cur, 1.0, n, dd["h"], dd["w"], dd["C"], dd["up"][:n])
-            eng._gemm(eng.dec[i], dd["up"][:n], dd["out"][:n], n, 2 * dd["h"], 2 * dd["w"], dd["C"], act=ACT_RELU6)
+            eng.gemm(eng.dec[i], dd["up"][:n], dd["out"][:n], n, 2 * dd["h"], 2 * dd["w"], dd["C"], act=ACT_RELU6)
             cur = dd["out"][:n]
             self.launches += 2
         ops.pred_sigmoid(cur, self.head[s], eng.pred_w, eng.pred_b, eng.bc, n * Hp * Wp, self.img[s], wt_head=eng.pred_wh,
@@ -798,14 +831,14 @@ class _Plan:
         """xs += fc2(GELU(fc1(LN(xs)))) (DTransformer.py:279-283,302-304): one fused kernel where supported.
         Returns True when the optional "x + merged" sum (sum_io += xs, sum_t = bf16) was fused into that kernel."""
         eng = self.eng
-        if eng.fuse_mlp and ops.mlp_fused_supported(C, 4 * C):
+        if d["mlp_fused"]:
             ops.mlp_fused(xs, P, C, 4 * C, blk["fc1_ln"].w, blk["fc1_ln"].bias, blk["fc2"].w, blk["fc2"].bias,
                           sum_io=sum_io, sum_t=sum_t)
             self.launches += 1
             return sum_io is not None
         else:
-            eng._gemm(blk["fc1_ln"], None, d["hid"], 1, P, 1, C, act=ACT_GELU, ln_frames=[xs])
-            eng._gemm(blk["fc2"], d["hid"], xs, 1, P, 1, 4 * C, out_f32=True, residual=xs)
+            eng.gemm(blk["fc1_ln"], None, d["hid"], 1, P, 1, C, act=ACT_GELU, ln_frames=[xs])
+            eng.gemm(blk["fc2"], d["hid"], xs, 1, P, 1, 4 * C, out_f32=True, residual=xs)
             self.launches += 2
         return False
 
@@ -815,27 +848,24 @@ class _Plan:
         d = self.lv[l]
         h, w, C = d["h"], d["w"], d["C"]
         P = B * h * w
-        nwin, ntok, D = d["nwin"], d["ntok"], eng.D
         feat = d["feat"].view(T, P, C)
         feat_t = d["feat_t"].view(T, P, C)
-        xs = d["xs"]
-        pre = "kv_fut" in d
+        xs, routes = d["xs"], d["routes"]
+        pre = KVPRE in routes
         if pre:
             # k | v of the (pre-attention) future neighbours, all frames at once per block
             # (one LayerNorm pass, then per block a 1x1 convolution over the [T*B, h, w, C] map on the TMA conv kernel)
             ops.layernorm(feat.view(T * P, C), T * P, C, d["ln_one"], d["ln_zero"], d["xn_all"])
             for i, blk in enumerate(eng.attn[l]):
-                eng._gemm(blk["kv_l"], d["xn_all"], d["kv_fut"][i].view(T * P, 2 * C), T * B, h, w, C)
+                eng.gemm(blk["kv_l"], d["xn_all"], d["kv_fut"][i].view(T * P, 2 * C), T * B, h, w, C)
             self.launches += 1 + len(eng.attn[l])
         for t in range(T):
             # past neighbours are already post-attention (updated in place), future ones are not: quirk Q1
             frames = [feat[t + o] if 0 <= t + o < T else None for o in eng.buf]      # None = all-zero map (Q4)
             qsrc = frames[eng.q_ind]
-            blk0 = eng.attn[l][0]
             # the first block (plain windows: every pixel belongs to exactly one window) of the fused-projection kernels
             # reads the query frame / shortcut straight from feat[t] and writes x: no copy of feat[t] into xs
-            direct0 = (qsrc is not None and blk0["tbl"] is not None
-                       and (C == 64 or pre or (eng.fuse_win256 and nwin >= eng.win256_min)))
+            direct0 = qsrc is not None and routes[0] in (WHOLE, KVPRE)
             if not direct0:
                 if qsrc is None:
                     xs.zero_()
@@ -843,80 +873,13 @@ class _Plan:
                     ops.cast(qsrc, xs)
                 self.launches += 1
             sum_done = False
-            for i, blk in enumerate(eng.attn[l]):
-                tm = d["tm"][i & 1]
+            for i, (blk, route) in enumerate(zip(eng.attn[l], routes)):
                 # the last block's fused MLP also does "x + merged[t]" (feat[t] += x, bf16 copy) -- bf16 engine only
-                last = i == len(eng.attn[l]) - 1 and eng.dtype != torch.float32
+                last = i == len(routes) - 1 and eng.dtype != torch.float32
                 sum_args = (feat[t], feat_t[t]) if last else (None, None)
                 fr = list(frames)
                 fr[eng.q_ind] = qsrc if (direct0 and i == 0) else xs
-                if blk["tbl"] is not None and pre:
-                    kv = [None] * D
-                    if t >= 1:
-                        kv[0] = d["kv_past"][(t - 1) & 1][:, i * 2 * C:(i + 1) * 2 * C]
-                    if t + 1 < T:
-                        kv[2] = d["kv_fut"][i, t + 1]
-                    ops.window_attention_fused_kvpre(fr[eng.q_ind], kv, eng.q_ind, tm.view(-1), nwin, C, eng.heads, blk["qkv"].w,
-                                                     blk["qkv"].bias, blk["tbl"], blk["proj"].w, blk["proj"].bias, xs)
-                    self.launches += 1
-                    sum_done = self._mlp(blk, d, xs, P, C, *sum_args)
-                    continue
-                if blk["tbl"] is not None:
-                    # one kernel for the attention half; C == 64 also projects and scatters into xs
-                    if C == 64 or (eng.fuse_win256 and nwin >= eng.win256_min):
-                        # C = 256: whole-window kernel (gather + LN once per window, projection + scatter fused) once
-                        # there are enough windows to fill the SMs with one CTA each; below that (a single sequence
-                        # has 35 level-3 windows) the per-head-group kernel's 4 CTAs per window finish sooner
-                        ops.window_attention_fused(fr, eng.q_ind, tm.view(-1), nwin, C, eng.heads, blk["qkv"].w,
-                                                   blk["qkv"].bias, blk["tbl"], blk["proj"].w, blk["proj"].bias, xs=xs)
-                        self.launches += 1
-                    else:
-                        ops.window_attention_fused(fr, eng.q_ind, tm.view(-1), nwin, C, eng.heads, blk["qkv"].w,
-                                                   blk["qkv"].bias, blk["tbl"], o_out=d["ob"])
-                        eng._gemm(blk["proj"], d["ob"], xs, 1, nwin * ntok, 1, C, epi=EPI_SCATTER, row_map=tm.view(-1))
-                        self.launches += 2
-                    sum_done = self._mlp(blk, d, xs, P, C, *sum_args)
-                    continue
-                if blk["qkv"] is not None:
-                    # fused: [window gather + LayerNorm + q/k/v projection] -> attention -> proj+scatter ->
-                    #        [LayerNorm + fc1 + GELU] -> fc2 + residual          (5 launches per block)
-                    M = nwin * D * ntok
-                    eng._gemm(blk["qkv"], None, d["qkv"], 1, M, 1, C, ln_frames=fr, ln_tok_map=tm.view(-1), ln_n_tok=ntok)
-                    ops.window_attention_mma_qkv(d["qkv"], blk["bias_mma"], nwin, ntok, D * ntok, eng.q_ind * ntok, C,
-                                                 eng.heads, d["ob"])
-                    eng._gemm(blk["proj"], d["ob"], xs, 1, nwin * ntok, 1, C, epi=EPI_SCATTER, row_map=tm.view(-1))
-                    sum_done = self._mlp(blk, d, xs, P, C, *sum_args)
-                    self.launches += 3
-                    continue
-                n_kvf = ntok
-                if blk["red"] is not None:
-                    # nwindow_size (DTransformer.py:172-175): q from the window's tokens, kv from the "feature reduction"
-                    # conv of every frame's window (raw tokens), then norm_kv
-                    rw, rb, n_kvf = blk["red"]
-                    ops.ln_gather([fr[eng.q_ind]], tm, nwin, ntok, C, blk["nq_g"], blk["nq_b"], d["qn"])
-                    ops.window_reduce(fr, tm.view(-1), nwin, ntok, C, n_kvf, rw, rb, d["kvr"])
-                    ops.layernorm(d["kvr"], nwin * D * n_kvf, C, blk["nkv_g"], blk["nkv_b"], d["kvn"])
-                    self.launches += 1
-                elif C in (64, 128, 256):
-                    ops.ln_gather_qkv(fr, eng.q_ind, tm, nwin, ntok, C, blk["nkv_g"], blk["nkv_b"], blk["nq_g"],
-                                      blk["nq_b"], d["kvn"], d["qn"])
-                    self.launches -= 1
-                else:
-                    ops.ln_gather([fr[eng.q_ind]], tm, nwin, ntok, C, blk["nq_g"], blk["nq_b"], d["qn"])
-                    ops.ln_gather(fr, tm, nwin, ntok, C, blk["nkv_g"], blk["nkv_b"], d["kvn"])
-                eng._gemm(blk["q"], d["qn"], d["qb"], 1, nwin * ntok, 1, C)
-                eng._gemm(blk["kv"], d["kvn"], d["kvb"], 1, nwin * D * n_kvf, 1, C)
-                if blk["bias_mma"] is not None:
-                    ops.window_attention_mma(d["qb"], d["kvb"], blk["bias_mma"], nwin, ntok, D * ntok, C, eng.heads,
-                                             d["ob"])
-                else:
-                    ops.window_attention(d["qb"], d["kvb"], blk["bias"], nwin, ntok, D * n_kvf, C, eng.heads, d["ob"])
-                # proj + window_reverse + crop + shortcut: x[pixel] += proj(o); uncovered pixels keep x
-                eng._gemm(blk["proj"], d["ob"], xs, 1, nwin * ntok, 1, C, epi=EPI_SCATTER, row_map=tm.view(-1))
-                ops.layernorm(xs, P, C, blk["n2_g"], blk["n2_b"], d["yn"])
-                eng._gemm(blk["fc1"], d["yn"], d["hid"], 1, P, 1, C, act=ACT_GELU)
-                eng._gemm(blk["fc2"], d["hid"], xs, 1, P, 1, 4 * C, out_f32=True, residual=xs)
-                self.launches += 9
+                sum_done = self._attention_block(route, i, blk, d, fr, t, sum_args)
             # x + merged[t], stored back in place (...V5.py:166-169), unless the last MLP kernel already did it
             if not sum_done:
                 ops.add(xs, feat[t], out_f32=feat[t], out_t=None if eng.dtype == torch.float32 else feat_t[t],
@@ -926,7 +889,71 @@ class _Plan:
                 # this frame is final: its k | v for every block of the next step (the "past" neighbour there)
                 xn_t = d["xn_all"][t * P:(t + 1) * P]      # (its pre-attention copy is not needed any more)
                 ops.layernorm(feat[t], P, C, d["ln_one"], d["ln_zero"], xn_t)
-                eng._gemm(eng.attn[l][0]["kv_all"], xn_t, d["kv_past"][t & 1], B, h, w, C)
+                eng.gemm(eng.attn[l][0]["kv_all"], xn_t, d["kv_past"][t & 1], B, h, w, C)
                 self.launches += 2
             if on_frame_done is not None:
                 on_frame_done(t)
+
+    def _attention_block(self, route, i, blk, d, fr, t, sum_args):
+        """Block ``i`` at frame ``t`` along its route, in place on xs (``fr``: its input frames).  Returns True when the
+        block's MLP kernel also did the "x + merged" sum of ``sum_args``."""
+        eng, C, nwin, ntok, D, xs = self.eng, d["C"], d["nwin"], d["ntok"], self.eng.D, d["xs"]
+        P = xs.shape[0]
+        tm = d["tm"][i & 1]
+        if route == UNFUSED:
+            n_kvf = ntok
+            if "red" in blk:
+                # nwindow_size (DTransformer.py:172-175): q from the window's tokens, kv from the "feature reduction"
+                # conv of every frame's window (raw tokens), then norm_kv
+                rw, rb, n_kvf = blk["red"]
+                ops.ln_gather([fr[eng.q_ind]], tm, nwin, ntok, C, blk["nq_g"], blk["nq_b"], d["qn"])
+                ops.window_reduce(fr, tm.view(-1), nwin, ntok, C, n_kvf, rw, rb, d["kvr"])
+                ops.layernorm(d["kvr"], nwin * D * n_kvf, C, blk["nkv_g"], blk["nkv_b"], d["kvn"])
+                self.launches += 3
+            elif C in (64, 128, 256):
+                ops.ln_gather_qkv(fr, eng.q_ind, tm, nwin, ntok, C, blk["nkv_g"], blk["nkv_b"], blk["nq_g"],
+                                  blk["nq_b"], d["kvn"], d["qn"])
+                self.launches += 1
+            else:
+                ops.ln_gather([fr[eng.q_ind]], tm, nwin, ntok, C, blk["nq_g"], blk["nq_b"], d["qn"])
+                ops.ln_gather(fr, tm, nwin, ntok, C, blk["nkv_g"], blk["nkv_b"], d["kvn"])
+                self.launches += 2
+            eng.gemm(blk["q"], d["qn"], d["qb"], 1, nwin * ntok, 1, C)
+            eng.gemm(blk["kv"], d["kvn"], d["kvb"], 1, nwin * D * n_kvf, 1, C)
+            if "bias_mma" in blk:
+                ops.window_attention_mma(d["qb"], d["kvb"], blk["bias_mma"], nwin, ntok, D * ntok, C, eng.heads, d["ob"])
+            else:
+                ops.window_attention(d["qb"], d["kvb"], blk["bias"], nwin, ntok, D * n_kvf, C, eng.heads, d["ob"])
+            # proj + window_reverse + crop + shortcut: x[pixel] += proj(o); uncovered pixels keep x
+            eng.gemm(blk["proj"], d["ob"], xs, 1, nwin * ntok, 1, C, epi=EPI_SCATTER, row_map=tm.view(-1))
+            ops.layernorm(xs, P, C, blk["n2_g"], blk["n2_b"], d["yn"])
+            eng.gemm(blk["fc1"], d["yn"], d["hid"], 1, P, 1, C, act=ACT_GELU)
+            eng.gemm(blk["fc2"], d["hid"], xs, 1, P, 1, 4 * C, out_f32=True, residual=xs)
+            self.launches += 7
+            return False
+        if route == KVPRE:
+            kv = [None] * D
+            if t >= 1:
+                kv[0] = d["kv_past"][(t - 1) & 1][:, i * 2 * C:(i + 1) * 2 * C]
+            if t + 1 < self.T:
+                kv[2] = d["kv_fut"][i, t + 1]
+            ops.window_attention_fused_kvpre(fr[eng.q_ind], kv, eng.q_ind, tm.view(-1), nwin, C, eng.heads, blk["qkv"].w,
+                                             blk["qkv"].bias, blk["tbl"], blk["proj"].w, blk["proj"].bias, xs)
+            self.launches += 1
+        elif route == WHOLE:
+            ops.window_attention_fused(fr, eng.q_ind, tm.view(-1), nwin, C, eng.heads, blk["qkv"].w, blk["qkv"].bias,
+                                       blk["tbl"], blk["proj"].w, blk["proj"].bias, xs=xs)
+            self.launches += 1
+        elif route == SPLIT:
+            ops.window_attention_fused(fr, eng.q_ind, tm.view(-1), nwin, C, eng.heads, blk["qkv"].w, blk["qkv"].bias,
+                                       blk["tbl"], o_out=d["ob"])
+            eng.gemm(blk["proj"], d["ob"], xs, 1, nwin * ntok, 1, C, epi=EPI_SCATTER, row_map=tm.view(-1))
+            self.launches += 2
+        else:   # QKV: [window gather + LayerNorm + q/k/v projection] -> attention -> proj + scatter
+            eng.gemm(blk["qkv"], None, d["qkv"], 1, nwin * D * ntok, 1, C, ln_frames=fr, ln_tok_map=tm.view(-1),
+                     ln_n_tok=ntok)
+            ops.window_attention_mma_qkv(d["qkv"], blk["bias_mma"], nwin, ntok, D * ntok, eng.q_ind * ntok, C, eng.heads,
+                                         d["ob"])
+            eng.gemm(blk["proj"], d["ob"], xs, 1, nwin * ntok, 1, C, epi=EPI_SCATTER, row_map=tm.view(-1))
+            self.launches += 3
+        return self._mlp(blk, d, xs, P, C, *sum_args)

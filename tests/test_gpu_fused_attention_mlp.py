@@ -728,7 +728,7 @@ def compact_table(sd, D, q_ind, heads):
 @pytest.mark.parametrize("D,q_ind,dilated", [(2, 0, False), (2, 1, True), (3, 1, False), (3, 0, True), (3, 2, False)])
 def test_reference_vs_oracle(D, q_ind, dilated):
     """The attention-half and MLP references without roundings (exact GELU), on the engine's folding
-    (engine.py:256-270) and compact tables rebuilt from relative_position_index, equal O.attention_block in float64."""
+    (engine.py:273-287) and compact tables rebuilt from relative_position_index, equal O.attention_block in float64."""
     C, heads, B, H, W = 64, 16, 2, 9, 16
     g = torch.Generator().manual_seed(D * 10 + q_ind + 100 * dilated)
     sd = _block_sd(C, heads, D, g)
