@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("BDE2VID_LIB") or os.path.join(_HERE, "libbde2vid_sm100.so")
 
 F32, BF16 = 0, 1
-ABI_VERSION = 2
+ABI_VERSION = 3
 ACT_NONE, ACT_RELU, ACT_RELU6, ACT_GELU, ACT_SIGMOID = 0, 1, 2, 3, 4
 EPI_STORE, EPI_LSTM, EPI_SCATTER, EPI_GRU_UR, EPI_GRU_OUT = 0, 1, 2, 3, 4
 ENGINE_SIMT, ENGINE_TCGEN05 = 0, 1
@@ -79,8 +79,6 @@ EXPORTS = {
     "bde_window_attention_fused_supported": (C.c_int, [C.c_int] * 4),
     "bde_window_attention_fused": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int]
                                    + [C.c_void_p] * 8),
-    "bde_window_attention_fused_kvpre": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int), C.c_int, C.c_int, C.c_void_p,
-                                                    C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 7),
     "bde_mlp_fused_supported": (C.c_int, [C.c_int, C.c_int]),
     "bde_mlp_fused": (C.c_int, [C.c_void_p, C.c_size_t, C.c_int, C.c_int] + [C.c_void_p] * 5),
     "bde_mlp_fused_sum": (C.c_int, [C.c_void_p, C.c_size_t, C.c_int, C.c_int] + [C.c_void_p] * 7),

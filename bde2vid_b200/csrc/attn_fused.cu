@@ -15,7 +15,6 @@
 #include "common.cuh"
 
 #include <cuda_fp16.h>
-#include <stdlib.h>
 // Ablation builds for tools/attn64_probe.sh (timing only, results are wrong): bit 0 = no bias-table loads, bit 1 = no MUFU.EX2
 // in the probabilities, 4 = skip the level-1 attention core altogether, 8 = no global gather (LayerNorm of zeros), 16 = no q/k/v
 // projection MMAs, 32 = no output projection + scatter.  0 in every shipped build.
@@ -47,10 +46,6 @@ struct FusedAttnParams {
   float* xs;                     // fp32 [P, C] += proj(attn)      (C == 64)
   __nv_bfloat16* o_out;          // bf16 [n_win * 49, C]           (C == 256)
   int n_win, D, q_slot, heads;
-  // whole-window kernel with precomputed neighbour k / v (kPre): bf16 [P, kv_ld[d]] rows = [k (C) | v (C)] of frame d,
-  // already offset to the block's columns; NULL = all-zero frame (k / v = bias).  Unused for the query slot.
-  const __nv_bfloat16* kvpre[8];
-  int kv_ld[8];
   long long* dbg;   // optional per-CTA phase cycle counters (8 slots per CTA), bring-up profiling
 };
 
@@ -148,13 +143,8 @@ __device__ __forceinline__ uint32_t ex2_h2(float lo, float hi) {
   return pack2_h(a, b);
 }
 
-// kPers (C == 64 only): ONE 512-thread CTA per SM; its two 256-thread halves walk the windows independently (named barriers)
-// on private token / q / k / v / output tiles, while the q|k|v weight slices, the bias table and the projection weights
-// are loaded ONCE per CTA into a region both halves share (the one-window form reloads those 65 KB for every window and
-// overlays the table on the token region to stay under half an SM's shared memory).
-template <int C, int HD, int NT, bool kPers = false>
+template <int C, int HD, int NT>
 struct FusedCfg {
-  static_assert(!kPers || C == 64, "the persistent form exists for C == 64 only");
   static constexpr int HG = 64 / HD;              // heads per CTA
   static constexpr int PX = C + 8;                // pitch (bf16 elements) of the LayerNorm'ed tokens and weight slices
   static constexpr int PQ = 72;                   // pitch of q / k / v / o tiles
@@ -170,26 +160,21 @@ struct FusedCfg {
   static constexpr int WP_BYTES = C == 64 ? 64 * PX * 2 : 0;
   // C == 64, one window per CTA: the bias table, the attention-output tile and the projection weights reuse the token /
   // weight region once the q, k, v projections are done (keeps the CTA under half an SM's shared memory)
-  static constexpr int A_BYTES = kPers ? (XN_BYTES > OS_BYTES ? XN_BYTES : OS_BYTES)
-                                 : C == 64 ? (XN_BYTES + W_BYTES > TBL_BYTES + OS_BYTES + WP_BYTES ? XN_BYTES + W_BYTES
-                                                                                                  : TBL_BYTES + OS_BYTES + WP_BYTES)
-                                           : XN_BYTES + W_BYTES + TBL_BYTES;
-  // regions relative to the SHARED base (kPers: start of shared memory, common to both halves)
-  static constexpr int OFF_W = kPers ? 0 : XN_BYTES;
-  static constexpr int OFF_TBL = kPers ? W_BYTES : (C == 64 ? 0 : XN_BYTES + W_BYTES);
-  static constexpr int OFF_WP = kPers ? W_BYTES + TBL_BYTES : TBL_BYTES + OS_BYTES;    // C == 64 only
-  static constexpr int SHARED_BYTES = kPers ? W_BYTES + TBL_BYTES + WP_BYTES : 0;
-  // regions relative to the HALF base (kPers: SHARED_BYTES + half * HALF_BYTES; otherwise the start of shared memory)
+  static constexpr int A_BYTES = C == 64 ? (XN_BYTES + W_BYTES > TBL_BYTES + OS_BYTES + WP_BYTES ? XN_BYTES + W_BYTES
+                                                                                               : TBL_BYTES + OS_BYTES + WP_BYTES)
+                                         : XN_BYTES + W_BYTES + TBL_BYTES;
   static constexpr int OFF_XN = 0;
-  static constexpr int OFF_OS = kPers ? 0 : TBL_BYTES;      // C == 64 only; kPers: over the (dead) token tile
+  static constexpr int OFF_W = XN_BYTES;
+  static constexpr int OFF_TBL = C == 64 ? 0 : XN_BYTES + W_BYTES;
+  static constexpr int OFF_OS = TBL_BYTES;                  // C == 64 only
+  static constexpr int OFF_WP = TBL_BYTES + OS_BYTES;       // C == 64 only
   static constexpr int OFF_Q = A_BYTES;
   static constexpr int OFF_K = OFF_Q + 64 * PQ * 2;
   static constexpr int OFF_V = OFF_K + NKEY * PQ * 2;
   static constexpr int OFF_COFF = OFF_V + XROWS * PQ * 2;   // int32 [NKEY]  byte offsets into a bias-table row block
   static constexpr int OFF_ROFF = OFF_COFF + NKEY * 4;      // int32 [64]
   static constexpr int OFF_PIX = OFF_ROFF + 256;            // int32 [64]
-  static constexpr int HALF_BYTES = OFF_PIX + 256;
-  static constexpr int SMEM = kPers ? SHARED_BYTES + 2 * HALF_BYTES : HALF_BYTES;
+  static constexpr int SMEM = OFF_PIX + 256;
 };
 
 // acc[mt][nt][4] += A[rows, C] (smem, pitch PX) * Wslice[64, C]^T (smem, pitch PX) for this warp's
@@ -223,40 +208,30 @@ __device__ __forceinline__ void warp_gemm(float (&acc)[MT][2][4], int n_mt, uint
   }
 }
 
-template <int C, int HD, int NT, bool kPers = false>
-__global__ void __launch_bounds__(kPers ? 2 * kThreadsF : kThreadsF, (C == 64 && !kPers) ? 2 : 1) attn_fused_kernel(const FusedAttnParams p) {
-  using Cfg = FusedCfg<C, HD, NT, kPers>;
+template <int C, int HD, int NT>
+__global__ void __launch_bounds__(kThreadsF, C == 64 ? 2 : 1) attn_fused_kernel(const FusedAttnParams p) {
+  using Cfg = FusedCfg<C, HD, NT>;
   constexpr int PX = Cfg::PX, PQ = Cfg::PQ, HG = Cfg::HG, KSTEPS = Cfg::KSTEPS, XROWS = Cfg::XROWS, NKEY = Cfg::NKEY;
   constexpr int NW = Cfg::NW;
   extern __shared__ __align__(16) uint8_t smem[];
   const uint32_t sb = (uint32_t)__cvta_generic_to_shared(smem);
-  // kPers: `half` = which 256-thread half of the CTA; tid / warp are relative to the half, smem_h / sb_h its private tiles
-  const int half = kPers ? (int)(threadIdx.x >> 8) : 0;
-  uint8_t* smem_h = smem + (kPers ? Cfg::SHARED_BYTES + half * Cfg::HALF_BYTES : 0);
-  const uint32_t sb_h = sb + (uint32_t)(kPers ? Cfg::SHARED_BYTES + half * Cfg::HALF_BYTES : 0);
-  __nv_bfloat16* xn = reinterpret_cast<__nv_bfloat16*>(smem_h + Cfg::OFF_XN);
+  __nv_bfloat16* xn = reinterpret_cast<__nv_bfloat16*>(smem + Cfg::OFF_XN);
   float* tbl_s = reinterpret_cast<float*>(smem + Cfg::OFF_TBL);
-  __nv_bfloat16* qs = reinterpret_cast<__nv_bfloat16*>(smem_h + Cfg::OFF_Q);
-  __nv_bfloat16* ks = reinterpret_cast<__nv_bfloat16*>(smem_h + Cfg::OFF_K);
-  __nv_bfloat16* vs = reinterpret_cast<__nv_bfloat16*>(smem_h + Cfg::OFF_V);
-  int* coff = reinterpret_cast<int*>(smem_h + Cfg::OFF_COFF);
-  int* roff = reinterpret_cast<int*>(smem_h + Cfg::OFF_ROFF);
-  int* pix_s = reinterpret_cast<int*>(smem_h + Cfg::OFF_PIX);
-  // barrier over the threads that share the tiles: the whole CTA, or (kPers) the 256 threads of this half
-  auto sync_tiles = [&]() {
-    if (kPers) asm volatile("bar.sync %0, 256;" ::"r"(1 + half) : "memory");
-    else __syncthreads();
-  };
+  __nv_bfloat16* qs = reinterpret_cast<__nv_bfloat16*>(smem + Cfg::OFF_Q);
+  __nv_bfloat16* ks = reinterpret_cast<__nv_bfloat16*>(smem + Cfg::OFF_K);
+  __nv_bfloat16* vs = reinterpret_cast<__nv_bfloat16*>(smem + Cfg::OFF_V);
+  int* coff = reinterpret_cast<int*>(smem + Cfg::OFF_COFF);
+  int* roff = reinterpret_cast<int*>(smem + Cfg::OFF_ROFF);
+  int* pix_s = reinterpret_cast<int*>(smem + Cfg::OFF_PIX);
 
-  const int tid = kPers ? (int)(threadIdx.x & 255) : (int)threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int tid = (int)threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int g = lane >> 2, t = lane & 3;
   const bool dbg = p.dbg != nullptr;
   const long long t_begin = dbg ? clock64() : 0;
   long long t_mark = t_begin, t_ln = 0, t_qkv = 0, t_tbl = 0, t_attn = 0;
   constexpr int NHG = C / 64;
-  const int hg = kPers ? 0 : (int)(blockIdx.x % NHG);
-  int w = kPers ? (int)blockIdx.x * 2 + half : (int)(blockIdx.x / NHG);
-  const int w_step = kPers ? (int)gridDim.x * 2 : 0;
+  const int hg = (int)(blockIdx.x % NHG);
+  const int w = (int)(blockIdx.x / NHG);
   const int n_kv = p.D * kTok;
   const int tbl_ld = p.D * kRel;
 
@@ -272,20 +247,7 @@ __global__ void __launch_bounds__(kPers ? 2 * kThreadsF : kThreadsF, (C == 64 &&
     cpa_commit();
   };
 #pragma unroll
-  for (int i = 0; i < NW; ++i) {
-    if (!kPers || i % 2 == half) load_w_slice(i, i);   // kPers: the halves share the loading (each thread waits for its own groups)
-  }
-  if (kPers) {
-    // bias table + projection weights, once per CTA (static data: before pdl_wait)
-    const float* src = p.tbl;
-    const int n16 = HG * tbl_ld / 4;
-    for (int i = (int)threadIdx.x; i < n16; i += 2 * kThreadsF) cpa16(sb + Cfg::OFF_TBL + (uint32_t)(i * 16), src + i * 4);
-    for (int i = (int)threadIdx.x; i < 64 * (C / 8); i += 2 * kThreadsF) {
-      const int r = i / (C / 8), ch = i - r * (C / 8);
-      cpa16(sb + Cfg::OFF_WP + (uint32_t)((r * PX + ch * 8) * 2), p.wproj + (size_t)r * C + ch * 8);
-    }
-    cpa_commit();
-  }
+  for (int i = 0; i < NW; ++i) load_w_slice(i, i);
 
   // ---- index tables -----------------------------------------------------------------------------------
   for (int n = tid; n < NKEY; n += kThreadsF) {
@@ -300,17 +262,9 @@ __global__ void __launch_bounds__(kPers ? 2 * kThreadsF : kThreadsF, (C == 64 &&
     const int a = tid / 7, b = tid - a * 7;
     roff[tid] = tid < kTok ? (a * 13 + b) * 4 : 0;
   }
-  if (kPers) {
-    cpa_wait<0>();
-    __syncthreads();   // weights, bias table and projection weights of BOTH halves' copies are in place
-  }
-  bool first_window = true;
-  if (kPers && w >= p.n_win) return;   // (an odd window count leaves the last half without work)
-  do {   // window loop; one window per CTA: a single pass
   if (tid < 64) pix_s[tid] = tid < kTok ? __ldg(p.tok_map + (size_t)w * kTok + tid) : -1;
-  sync_tiles();
-  if (first_window) pdl_wait();   // everything above is static data; the frames below were written by the previous kernel of the chain
-  first_window = false;
+  __syncthreads();
+  pdl_wait();   // everything above is static data; the frames below were written by the previous kernel of the chain
 
   // ---- gather + LayerNorm: 8 lanes per token, 4 tokens per warp pass ----------------------------------
   // The loads of NB passes are issued together (independent global reads in flight) before any of them is reduced.
@@ -393,17 +347,17 @@ __global__ void __launch_bounds__(kPers ? 2 * kThreadsF : kThreadsF, (C == 64 &&
   if (dbg) { const long long c = clock64(); t_ln = c - t_mark; t_mark = c; }
   // ---- q, k, v projections (mma.sync): warp = (n-tile pair, m half) --------------------------------------
   const int npair = warp & 3, mh = warp >> 2;
-  const uint32_t xn_u32 = sb_h + Cfg::OFF_XN;
+  const uint32_t xn_u32 = sb + Cfg::OFF_XN;
   constexpr int MTK = (KSTEPS + 1) / 2;  // k / v m-tiles per warp
   if (NW == 3) {  // all three weight slices were loaded up front: one barrier covers them and the LayerNorm'ed tokens
-    if (!kPers) cpa_wait<0>();
-    sync_tiles();
+    cpa_wait<0>();
+    __syncthreads();
   }
   for (int which = 0; which < ((BDE_ATTN_PROBE & 16) ? 0 : 3); ++which) {
     if (NW != 3) {
       // slices were committed in order: wait until slice `which` has landed
       if (which == 2) cpa_wait<0>(); else cpa_wait<1>();
-      sync_tiles();  // slice + (first pass) the LayerNorm'ed tokens visible to every warp
+      __syncthreads();  // slice + (first pass) the LayerNorm'ed tokens visible to every warp
     }
     const uint32_t w_base = sb + Cfg::OFF_W + (uint32_t)((which % NW) * 64 * PX * 2);
     const float* bsrc = p.bqkv + which * C + hg * 64 + npair * 16 + 2 * t;
@@ -449,15 +403,15 @@ __global__ void __launch_bounds__(kPers ? 2 * kThreadsF : kThreadsF, (C == 64 &&
       }
     }
     if (which + NW < 3) {
-      sync_tiles();  // every warp is done reading buffer which % NW
+      __syncthreads();  // every warp is done reading buffer which % NW
       load_w_slice(which + NW, which % NW);
     }
   }
-  sync_tiles();  // q, k, v complete; the token / weight region is free
+  __syncthreads();  // q, k, v complete; the token / weight region is free
   if (dbg) { const long long c = clock64(); t_qkv = c - t_mark; t_mark = c; }
 
   // ---- bias table (+ projection weights) -> smem ------------------------------------------------------------
-  if (!kPers) {
+  {
     const float* src = p.tbl + (size_t)hg * HG * tbl_ld;
     const int n16 = HG * tbl_ld / 4;  // 16-byte chunks (HG * D * 169 floats; multiple of 4 because HG is)
     for (int i = tid; i < n16; i += kThreadsF) cpa16(sb + Cfg::OFF_TBL + (uint32_t)(i * 16), src + i * 4);
@@ -469,7 +423,7 @@ __global__ void __launch_bounds__(kPers ? 2 * kThreadsF : kThreadsF, (C == 64 &&
     }
     cpa_commit();
     cpa_wait<0>();
-    sync_tiles();
+    __syncthreads();
   }
 
   if (dbg) { const long long c = clock64(); t_tbl = c - t_mark; t_mark = c; }
@@ -477,10 +431,10 @@ __global__ void __launch_bounds__(kPers ? 2 * kThreadsF : kThreadsF, (C == 64 &&
   // head_dim 4: the 49th query row would cost a whole tile per head, so the normal units cover rows 0..47 and one
   // "special" unit packs row 48 of all 16 heads into a single tile (tile row = head; the query fragment carries only
   // that head's 4 channels, the key fragment all 64, so each row still sees its own head's dot product).
-  const uint32_t vs_u32 = sb_h + Cfg::OFF_V;
+  const uint32_t vs_u32 = sb + Cfg::OFF_V;
   const uint32_t tbl_u32 = sb + Cfg::OFF_TBL;
-  const uint32_t coff_u32 = sb_h + Cfg::OFF_COFF;
-  __nv_bfloat16* os = reinterpret_cast<__nv_bfloat16*>(smem_h + Cfg::OFF_OS);  // C == 64 only
+  const uint32_t coff_u32 = sb + Cfg::OFF_COFF;
+  __nv_bfloat16* os = reinterpret_cast<__nv_bfloat16*>(smem + Cfg::OFF_OS);  // C == 64 only
   constexpr int MTN = HD == 4 ? 3 : 4;                 // query tiles per head handled by normal units
   constexpr int NUNITS = HG * MTN;
   constexpr uint32_t kOnes = 0x3C003C00u;              // fp16x2 (1, 1)
@@ -789,9 +743,9 @@ __global__ void __launch_bounds__(kPers ? 2 * kThreadsF : kThreadsF, (C == 64 &&
           sc[i][hrow][n] = pix >= 0 ? *(reinterpret_cast<const float2*>(shortcut + (size_t)pix * C + npair * 16 + n * 8 + 2 * t))
                                     : make_float2(0.f, 0.f);
       }
-    sync_tiles();
+    __syncthreads();
     float acc[2][2][4];
-    warp_gemm<C, PQ, 2>(acc, 2, sb_h + Cfg::OFF_OS, [&](int i, int r) { return (mh * 2 + i) * 16 + r; }, sb + Cfg::OFF_WP, npair, lane);
+    warp_gemm<C, PQ, 2>(acc, 2, sb + Cfg::OFF_OS, [&](int i, int r) { return (mh * 2 + i) * 16 + r; }, sb + Cfg::OFF_WP, npair, lane);
     // note: os has pitch PQ == PX for C == 64, so the same routine serves both operands
 #pragma unroll
     for (int i = 0; i < 2; ++i) {
@@ -813,9 +767,7 @@ __global__ void __launch_bounds__(kPers ? 2 * kThreadsF : kThreadsF, (C == 64 &&
       }
     }
   }
-  if (kPers) sync_tiles();   // the next window overwrites pix_s and the token tile that the projection above reads
-  } while (kPers && (w += w_step) < p.n_win);
-  if (dbg && tid == 0 && !kPers) {
+  if (dbg && tid == 0) {
     long long* o = p.dbg + (size_t)blockIdx.x * 8;
     const long long c = clock64();
     o[0] = c - t_begin; o[1] = t_ln; o[2] = 0; o[3] = t_qkv; o[4] = t_tbl; o[5] = t_attn; o[6] = c - t_mark;
@@ -836,484 +788,6 @@ int launch_fused(const FusedAttnParams& p, cudaStream_t s) {
   const cudaError_t le = launch_pdl(kern, (unsigned)(p.n_win * (C / 64)), (unsigned)kThreadsF, (size_t)Cfg::SMEM, s, 1, q);
   BDE_REQUIRE(le == cudaSuccess, "bde_window_attention_fused: launch: %s", cudaGetErrorString(le));
   return check_launch("attn_fused_kernel");
-}
-
-// C == 64, persistent form: one 512-thread CTA per SM, two halves walking the windows (see FusedCfg<.., kPers = true>)
-template <int NT>
-int launch_fused_pers(const FusedAttnParams& p, cudaStream_t s) {
-  using Cfg = FusedCfg<64, 4, NT, true>;
-  auto kern = attn_fused_kernel<64, 4, NT, true>;
-  if (first_use_on_device((const void*)kern)) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM);
-    BDE_REQUIRE(e == cudaSuccess, "bde_window_attention_fused: smem attribute (%d bytes): %s", Cfg::SMEM, cudaGetErrorString(e));
-  }
-  FusedAttnParams q = p;
-  q.dbg = nullptr;
-  const int n_sm = device_sm_count();
-  const int ctas = (p.n_win + 1) / 2 < n_sm ? (p.n_win + 1) / 2 : n_sm;
-  const cudaError_t le = launch_pdl(kern, (unsigned)ctas, (unsigned)(2 * kThreadsF), (size_t)Cfg::SMEM, s, 1, q);
-  BDE_REQUIRE(le == cudaSuccess, "bde_window_attention_fused: launch (persistent): %s", cudaGetErrorString(le));
-  return check_launch("attn_fused_kernel (persistent)");
-}
-
-
-// =====================================================================================================================
-// C = 256 (16 heads of 16 channels), whole-window form: ONE 512-thread CTA per window walks the four 64-column head
-// groups, so the gather + LayerNorm of the window's D x 49 tokens is done once (the per-head-group kernel above redoes
-// it in each of its 4 CTAs), sixteen warps instead of eight hide the mma.sync / shared-memory latencies, and the output
-// projection + window_reverse + shortcut (DTransformer.py:204, 294-299) run in the same kernel on the [49 x 256]
-// attention output that never leaves shared memory -- the separate proj GEMM launch and its bf16 round trip are gone.
-// Weights stream through two [64 x 128] half-slice buffers (cp.async ping-pong): 12 q/k/v slices + 4 proj slices.
-// =====================================================================================================================
-constexpr int kThreadsW = 512;
-
-template <int NT, bool kPre = false>
-struct WinCfg {
-  static constexpr int C = 256, HD = 16, HG = 4, NHG = 4;
-  static constexpr int PX = C + 8;                // LayerNorm'ed tokens / attention-output pitch (bf16 elements)
-  static constexpr int PH = 128 + 8;              // weight half-slice pitch
-  static constexpr int PQ = 72;
-  static constexpr int KSTEPS = (NT + 1) / 2;
-  static constexpr int XROWS = KSTEPS * 16;
-  static constexpr int NKEY = NT * 8;
-  static constexpr int DMAX = NT <= 7 ? 1 : (NT <= 13 ? 2 : 3);
-  static constexpr int XNROWS = kPre ? 64 : XROWS;                // LayerNorm'ed token rows staged (kPre: query frame only)
-  static constexpr int NBUF = kPre ? 5 : 2;                       // weight half-slice buffers (prefetch distance NBUF - 1)
-  static constexpr int OFF_XN = 0;
-  static constexpr int OFF_WB = OFF_XN + XNROWS * PX * 2;         // NBUF x [64 x PH]
-  static constexpr int OFF_Q = OFF_WB + NBUF * 64 * PH * 2;
-  static constexpr int OFF_K = OFF_Q + 64 * PQ * 2;
-  static constexpr int OFF_V = OFF_K + NKEY * PQ * 2;
-  static constexpr int OFF_O = OFF_V + XROWS * PQ * 2;            // [64 x PX] attention output of all heads
-  static constexpr int OFF_TBL = OFF_O + 64 * PX * 2;             // HG x DMAX x 169 floats of the current head group
-  static constexpr int OFF_COFF = OFF_TBL + HG * DMAX * kRel * 4;
-  static constexpr int OFF_ROFF = OFF_COFF + NKEY * 4;
-  static constexpr int OFF_PIX = OFF_ROFF + 256;
-  static constexpr int SMEM = OFF_PIX + 256;
-  static_assert(SMEM <= 232448, "shared memory budget");
-};
-
-// acc[i][n][4] += A[rows, k0 .. k0 + 128) (smem, pitch PX) * Whalf[64, 128]^T (smem, pitch PH)
-// Software pipelined: the ldmatrix loads of k step kk + 1 are issued before the MMAs of step kk (the profile of the
-// straight loop showed the HMMAs stalled on the short scoreboard, i.e. on their own fragments).
-template <int PX, int PH, int MT, typename RowFn>
-__device__ __forceinline__ void warp_gemm_half(float (&acc)[MT][2][4], int n_mt, uint32_t a_base, RowFn a_row, int k0, uint32_t w_base,
-                                               int npair, int lane) {
-  const int bm = lane >> 3;
-  const uint32_t b_addr0 = w_base + (uint32_t)(((npair * 16 + (bm >> 1) * 8 + (lane & 7)) * PH + (bm & 1) * 8) * 2);
-  uint32_t a_addr[MT];
-#pragma unroll
-  for (int i = 0; i < MT; ++i) a_addr[i] = a_base + (uint32_t)((a_row(i, lane & 15) * PX + k0 + (lane >> 4) * 8) * 2);
-  uint32_t b[2][4], a[2][MT][4];
-  ldsm_x4(b[0], b_addr0);
-#pragma unroll
-  for (int i = 0; i < MT; ++i)
-    if (i < n_mt) ldsm_x4(a[0][i], a_addr[i]);
-#pragma unroll
-  for (int kk = 0; kk < 8; ++kk) {
-    const int cur = kk & 1, nxt = cur ^ 1;
-    if (kk + 1 < 8) {
-      ldsm_x4(b[nxt], b_addr0 + (uint32_t)((kk + 1) * 32));
-#pragma unroll
-      for (int i = 0; i < MT; ++i)
-        if (i < n_mt) ldsm_x4(a[nxt][i], a_addr[i] + (uint32_t)((kk + 1) * 32));
-    }
-#pragma unroll
-    for (int i = 0; i < MT; ++i) {
-      if (i < n_mt) {
-        mma16816(acc[i][0], a[cur][i], b[cur][0], b[cur][1]);
-        mma16816(acc[i][1], a[cur][i], b[cur][2], b[cur][3]);
-      }
-    }
-  }
-}
-
-// kPre: the k / v rows of the D - 1 neighbour frames were produced ahead of the chain by LayerNorm-GEMM launches on the
-// tcgen05 engine (they do not depend on the running x) and are only gathered here; the kernel then normalises and
-// projects just the 49 query-frame tokens (q, k, v), i.e. 64 instead of 160 rows per weight slice.
-template <int NT, bool kPre>
-__global__ void __launch_bounds__(kThreadsW, 1) attn_win256_kernel(const FusedAttnParams p) {
-  using Cfg = WinCfg<NT, kPre>;
-  constexpr int XNROWS = Cfg::XNROWS;
-  constexpr int C = Cfg::C, HD = Cfg::HD, HG = Cfg::HG, PX = Cfg::PX, PH = Cfg::PH, PQ = Cfg::PQ;
-  constexpr int KSTEPS = Cfg::KSTEPS, XROWS = Cfg::XROWS, NKEY = Cfg::NKEY, NBUF = Cfg::NBUF;
-  extern __shared__ __align__(16) uint8_t smem[];
-  const uint32_t sb = (uint32_t)__cvta_generic_to_shared(smem);
-  __nv_bfloat16* xn = reinterpret_cast<__nv_bfloat16*>(smem + Cfg::OFF_XN);
-  __nv_bfloat16* qs = reinterpret_cast<__nv_bfloat16*>(smem + Cfg::OFF_Q);
-  __nv_bfloat16* ks = reinterpret_cast<__nv_bfloat16*>(smem + Cfg::OFF_K);
-  __nv_bfloat16* vs = reinterpret_cast<__nv_bfloat16*>(smem + Cfg::OFF_V);
-  __nv_bfloat16* os = reinterpret_cast<__nv_bfloat16*>(smem + Cfg::OFF_O);
-  int* coff = reinterpret_cast<int*>(smem + Cfg::OFF_COFF);
-  int* roff = reinterpret_cast<int*>(smem + Cfg::OFF_ROFF);
-  int* pix_s = reinterpret_cast<int*>(smem + Cfg::OFF_PIX);
-
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int g = lane >> 2, t = lane & 3;
-  const int w = blockIdx.x;
-  const int n_kv = p.D * kTok;
-  const int tbl_ld = p.D * kRel;
-
-  // weight half-slice hs (0 .. 31): slice = hs / 2 (q, k, v of head group 0..3, then the 4 proj slices), K half = hs & 1
-  long long t_ln = 0, t_gemm = 0, t_gather = 0, t_tbl = 0, t_attn = 0;
-  const bool dbg = p.dbg != nullptr;
-  const long long t_begin = dbg ? clock64() : 0;
-  auto load_half = [&](int hs) {
-    const int sl = hs >> 1, half = hs & 1;
-    const __nv_bfloat16* src;
-    if (sl < 12) {
-      const int hg = sl / 3, which = sl - hg * 3;
-      src = p.wqkv + (size_t)(which * C + hg * 64) * C + half * 128;
-    } else {
-      src = p.wproj + (size_t)((sl - 12) * 64) * C + half * 128;
-    }
-    const uint32_t dst = sb + Cfg::OFF_WB + (uint32_t)((hs % NBUF) * 64 * PH * 2);
-    for (int i = tid; i < 64 * 16; i += kThreadsW) {
-      const int r = i >> 4, ch = i & 15;
-      cpa16(dst + (uint32_t)((r * PH + ch * 8) * 2), src + (size_t)r * C + ch * 8);
-    }
-    cpa_commit();
-  };
-#pragma unroll
-  for (int i = 0; i < NBUF - 1; ++i) load_half(i);
-
-  // ---- index tables -----------------------------------------------------------------------------------
-  for (int n = tid; n < NKEY; n += kThreadsW) {
-    int v = 0;
-    if (n < n_kv) {
-      const int d = n / kTok, r = n - d * kTok, a = r / 7, b = r - a * 7;
-      v = d * kRel + (6 - a) * 13 + (6 - b);
-    }
-    coff[n] = v * 4;
-  }
-  if (tid < 64) {
-    const int a = tid / 7, b = tid - a * 7;
-    roff[tid] = tid < kTok ? (a * 13 + b) * 4 : 0;
-    pix_s[tid] = tid < kTok ? __ldg(p.tok_map + (size_t)w * kTok + tid) : -1;
-  }
-  __syncthreads();
-  pdl_wait();   // the frames (and the precomputed k | v) below were written by earlier kernels of the chain
-
-  // ---- gather + LayerNorm, once per window: 8 lanes per token, 64 tokens per pass ---------------------
-  {
-    const int j = lane & 7, sub = lane >> 3;
-    for (int pass = 0; pass * 64 < XNROWS; ++pass) {
-      const int n = pass * 64 + warp * 4 + sub;
-      if (n >= XNROWS) continue;   // uniform per 4-token group; XNROWS is a multiple of 16
-      const float* src = nullptr;
-      if (kPre ? n < kTok : n < n_kv) {
-        const int d = kPre ? p.q_slot : n / kTok, tok = kPre ? n : n - (n / kTok) * kTok;
-        const int pix = pix_s[tok];
-        const float* fr = p.frames[0];
-#pragma unroll
-        for (int q = 1; q < 8; ++q) fr = (d == q) ? p.frames[q] : fr;
-        if (fr != nullptr && pix >= 0) src = fr + (size_t)pix * C + j * 8;
-      }
-      float v[4][8];
-      float sum = 0.f;
-#pragma unroll
-      for (int kb = 0; kb < 4; ++kb) {
-        if (src != nullptr) {
-          const float4 t0 = *(reinterpret_cast<const float4*>(src + kb * 64));
-          const float4 t1 = *(reinterpret_cast<const float4*>(src + kb * 64 + 4));
-          v[kb][0] = t0.x; v[kb][1] = t0.y; v[kb][2] = t0.z; v[kb][3] = t0.w;
-          v[kb][4] = t1.x; v[kb][5] = t1.y; v[kb][6] = t1.z; v[kb][7] = t1.w;
-        } else {
-#pragma unroll
-          for (int e = 0; e < 8; ++e) v[kb][e] = 0.f;
-        }
-#pragma unroll
-        for (int e = 0; e < 8; ++e) sum += v[kb][e];
-      }
-      sum += __shfl_xor_sync(0xffffffffu, sum, 1);
-      sum += __shfl_xor_sync(0xffffffffu, sum, 2);
-      sum += __shfl_xor_sync(0xffffffffu, sum, 4);
-      const float mean = sum / (float)C;
-      float sq = 0.f;
-#pragma unroll
-      for (int kb = 0; kb < 4; ++kb)
-#pragma unroll
-        for (int e = 0; e < 8; ++e) {
-          const float dlt = v[kb][e] - mean;
-          v[kb][e] = dlt;
-          sq += dlt * dlt;
-        }
-      sq += __shfl_xor_sync(0xffffffffu, sq, 1);
-      sq += __shfl_xor_sync(0xffffffffu, sq, 2);
-      sq += __shfl_xor_sync(0xffffffffu, sq, 4);
-      const float rstd = 1.0f / sqrtf(sq / (float)C + 1e-5f);
-#pragma unroll
-      for (int kb = 0; kb < 4; ++kb) {
-        uint4 pk;
-        pk.x = pack2(v[kb][0] * rstd, v[kb][1] * rstd);
-        pk.y = pack2(v[kb][2] * rstd, v[kb][3] * rstd);
-        pk.z = pack2(v[kb][4] * rstd, v[kb][5] * rstd);
-        pk.w = pack2(v[kb][6] * rstd, v[kb][7] * rstd);
-        *reinterpret_cast<uint4*>(xn + (size_t)n * PX + kb * 64 + j * 8) = pk;
-      }
-    }
-  }
-
-  if (dbg) t_ln = clock64() - t_begin;
-  const int npair = warp & 3, mq = warp >> 2;
-  const uint32_t xn_u32 = sb + Cfg::OFF_XN, os_u32 = sb + Cfg::OFF_O;
-  const uint32_t vs_u32 = sb + Cfg::OFF_V, tbl_u32 = sb + Cfg::OFF_TBL, coff_u32 = sb + Cfg::OFF_COFF;
-  constexpr int MTK = (KSTEPS + 3) / 4;   // k / v m-tiles per warp (4 m groups)
-  constexpr uint32_t kOnes = 0x3C003C00u;
-  constexpr float kLog2e = 1.4426950408889634f;
-  int hs = 0;   // next half-slice to consume (its load has been issued)
-
-  // one weight slice = two half-slices: wait for the half, release the other buffer to the next load, accumulate
-  auto slice_gemm = [&](auto& acc, int n_mt, uint32_t a_base, auto a_row) {
-#pragma unroll
-    for (int half = 0; half < 2; ++half, ++hs) {
-      cpa_wait<NBUF - 2>();                  // all but the NBUF - 2 youngest groups are complete: half-slice hs landed
-      __syncthreads();                       // ... for every thread; every warp is done with buffer (hs - 1) % NBUF
-      if (hs + NBUF - 1 < 32) load_half(hs + NBUF - 1); else cpa_commit();   // (empty group keeps the count uniform)
-      warp_gemm_half<PX, PH, (int)(sizeof(acc) / sizeof(acc[0]))>(acc, n_mt, a_base, a_row, half * 128,
-                                                                   sb + Cfg::OFF_WB + (uint32_t)((hs % NBUF) * 64 * PH * 2), npair, lane);
-    }
-  };
-
-  if (kPre) {
-    // rows past the last key: finite zeros (they are masked in the scores / multiplied by p = 0)
-    for (int i = tid; i < (NKEY - n_kv) * 64; i += kThreadsW) ks[(n_kv + i / 64) * PQ + (i & 63)] = __float2bfloat16_rn(0.f);
-    for (int i = tid; i < (XROWS - n_kv) * 64; i += kThreadsW) vs[(n_kv + i / 64) * PQ + (i & 63)] = __float2bfloat16_rn(0.f);
-  }
-  for (int hg = 0; hg < Cfg::NHG; ++hg) {
-    long long t0 = dbg ? clock64() : 0;
-    if (kPre) {
-      // ---- neighbour frames: gather the precomputed k / v columns of this head group (v: bf16 -> fp16) -------------------
-      if (hg > 0) __syncthreads();   // every warp is done with the previous group's k / v tiles
-      const int per = kTok * (p.D - 1);
-      for (int i = tid; i < 2 * per * 8; i += kThreadsW) {
-        const int c8 = i & 7, rest = i >> 3;
-        const int which = rest / per, ti = rest - which * per;          // 0 = k, 1 = v
-        const int dd = ti / kTok, tok = ti - dd * kTok;
-        const int d = dd < p.q_slot ? dd : dd + 1;
-        const int pix = pix_s[tok];
-        const __nv_bfloat16* src = p.kvpre[0];
-        int ld = p.kv_ld[0];
-#pragma unroll
-        for (int q = 1; q < 8; ++q) {
-          src = (d == q) ? p.kvpre[q] : src;
-          ld = (d == q) ? p.kv_ld[q] : ld;
-        }
-        uint4 val;
-        if (src != nullptr && pix >= 0) {
-          val = __ldg(reinterpret_cast<const uint4*>(src + (size_t)pix * ld + which * C + hg * 64 + c8 * 8));
-        } else {   // zero token: LayerNorm(0) = 0 -> k / v = folded bias
-          const float* bs = p.bqkv + (1 + which) * C + hg * 64 + c8 * 8;
-          val.x = pack2(__ldg(bs + 0), __ldg(bs + 1)); val.y = pack2(__ldg(bs + 2), __ldg(bs + 3));
-          val.z = pack2(__ldg(bs + 4), __ldg(bs + 5)); val.w = pack2(__ldg(bs + 6), __ldg(bs + 7));
-        }
-        if (which == 1) {
-          uint32_t wv[4] = {val.x, val.y, val.z, val.w};
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            const float2 f2 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&wv[e]));
-            wv[e] = pack2_hs(f2.x, f2.y);
-          }
-          val = make_uint4(wv[0], wv[1], wv[2], wv[3]);
-        }
-        *reinterpret_cast<uint4*>((which == 0 ? ks : vs) + (d * kTok + tok) * PQ + c8 * 8) = val;
-      }
-    }
-    if (dbg) { const long long t1 = clock64(); t_gather += t1 - t0; t0 = t1; }
-    // ---- q, k, v projections of this head group --------------------------------------------------------------------
-    for (int which = 0; which < 3; ++which) {
-      const float* bsrc = p.bqkv + which * C + hg * 64 + npair * 16 + 2 * t;
-      const float2 bia0 = __ldg(reinterpret_cast<const float2*>(bsrc));
-      const float2 bia1 = __ldg(reinterpret_cast<const float2*>(bsrc + 8));
-      if (which == 0) {
-        float acc[1][2][4];
-        acc[0][0][0] = acc[0][0][1] = acc[0][0][2] = acc[0][0][3] = acc[0][1][0] = acc[0][1][1] = acc[0][1][2] = acc[0][1][3] = 0.f;
-        const int qrow0 = p.q_slot * kTok;
-        slice_gemm(acc, 1, xn_u32, [&](int i, int r) { return kPre ? mq * 16 + r : min(qrow0 + mq * 16 + r, XNROWS - 1); });
-        const int r0 = mq * 16 + g;
-#pragma unroll
-        for (int n = 0; n < 2; ++n) {
-          const float2 bb = n == 0 ? bia0 : bia1;
-          const int col = npair * 16 + n * 8 + 2 * t;
-          *reinterpret_cast<uint32_t*>(qs + r0 * PQ + col) = pack2(acc[0][n][0] + bb.x, acc[0][n][1] + bb.y);
-          *reinterpret_cast<uint32_t*>(qs + (r0 + 8) * PQ + col) = pack2(acc[0][n][2] + bb.x, acc[0][n][3] + bb.y);
-        }
-      } else if (kPre) {
-        // k / v of the query frame's own 49 tokens (XN rows 0..63) -> tile rows q_slot * 49 + token
-        float acc[1][2][4];
-        acc[0][0][0] = acc[0][0][1] = acc[0][0][2] = acc[0][0][3] = acc[0][1][0] = acc[0][1][1] = acc[0][1][2] = acc[0][1][3] = 0.f;
-        slice_gemm(acc, 1, xn_u32, [&](int i, int r) { return mq * 16 + r; });
-        __nv_bfloat16* dstm = which == 1 ? ks : vs;
-        const int tok0 = mq * 16 + g, base = p.q_slot * kTok;
-#pragma unroll
-        for (int n = 0; n < 2; ++n) {
-          const float2 bb = n == 0 ? bia0 : bia1;
-          const int col = npair * 16 + n * 8 + 2 * t;
-          const float v00 = acc[0][n][0] + bb.x, v01 = acc[0][n][1] + bb.y, v10 = acc[0][n][2] + bb.x, v11 = acc[0][n][3] + bb.y;
-          if (tok0 < kTok) *reinterpret_cast<uint32_t*>(dstm + (base + tok0) * PQ + col) = which == 1 ? pack2(v00, v01) : pack2_hs(v00, v01);
-          if (tok0 + 8 < kTok)
-            *reinterpret_cast<uint32_t*>(dstm + (base + tok0 + 8) * PQ + col) = which == 1 ? pack2(v10, v11) : pack2_hs(v10, v11);
-        }
-      } else {
-        float acc[MTK][2][4];
-#pragma unroll
-        for (int i = 0; i < MTK; ++i)
-#pragma unroll
-          for (int n = 0; n < 2; ++n) acc[i][n][0] = acc[i][n][1] = acc[i][n][2] = acc[i][n][3] = 0.f;
-        const int mt0 = mq * MTK;
-        const int n_mt = max(0, min(MTK, KSTEPS - mt0));
-        slice_gemm(acc, n_mt, xn_u32, [&](int i, int r) { return (mt0 + i) * 16 + r; });
-        __nv_bfloat16* dstm = which == 1 ? ks : vs;
-        const int row_lim = which == 1 ? NKEY : XROWS;
-#pragma unroll
-        for (int i = 0; i < MTK; ++i) {
-          if (i < n_mt) {
-            const int r0 = (mt0 + i) * 16 + g;
-#pragma unroll
-            for (int n = 0; n < 2; ++n) {
-              const float2 bb = n == 0 ? bia0 : bia1;
-              const int col = npair * 16 + n * 8 + 2 * t;
-              const float v00 = acc[i][n][0] + bb.x, v01 = acc[i][n][1] + bb.y, v10 = acc[i][n][2] + bb.x, v11 = acc[i][n][3] + bb.y;
-              if (r0 < row_lim) *reinterpret_cast<uint32_t*>(dstm + r0 * PQ + col) = which == 1 ? pack2(v00, v01) : pack2_hs(v00, v01);
-              if (r0 + 8 < row_lim)
-                *reinterpret_cast<uint32_t*>(dstm + (r0 + 8) * PQ + col) = which == 1 ? pack2(v10, v11) : pack2_hs(v10, v11);
-            }
-          }
-        }
-      }
-    }
-    if (dbg) { const long long t1 = clock64(); t_gemm += t1 - t0; t0 = t1; }
-    // ---- bias table of this head group -> smem; q, k, v visible ----------------------------------------------------
-    {
-      const float* src = p.tbl + (size_t)hg * HG * tbl_ld;
-      const int n16 = HG * tbl_ld / 4;
-      for (int i = tid; i < n16; i += kThreadsW) cpa16(sb + Cfg::OFF_TBL + (uint32_t)(i * 16), src + i * 4);
-      cpa_commit();
-      cpa_wait<0>();   // also covers the weight half-slice that is in flight (needed next anyway)
-      __syncthreads();
-    }
-    if (dbg) { const long long t1 = clock64(); t_tbl += t1 - t0; t0 = t1; }
-    // ---- attention: warp = (head of the group, 16-row query tile); scores stay in registers ---------------------------
-    {
-      const int hl = warp >> 2, mt = warp & 3;
-      const int row0 = mt * 16 + g, row1 = row0 + 8;
-      float s[NT][4];
-      const uint32_t r0a = tbl_u32 + (uint32_t)(hl * tbl_ld * 4 + roff[row0]);
-      const uint32_t r1a = tbl_u32 + (uint32_t)(hl * tbl_ld * 4 + roff[row1]);
-      uint32_t qa[4];
-      {
-        const __nv_bfloat16* q0 = qs + row0 * PQ + hl * HD;
-        const __nv_bfloat16* q1 = qs + row1 * PQ + hl * HD;
-        qa[0] = *reinterpret_cast<const uint32_t*>(q0 + 2 * t);
-        qa[1] = *reinterpret_cast<const uint32_t*>(q1 + 2 * t);
-        qa[2] = *reinterpret_cast<const uint32_t*>(q0 + 2 * t + 8);
-        qa[3] = *reinterpret_cast<const uint32_t*>(q1 + 2 * t + 8);
-      }
-#pragma unroll
-      for (int j = 0; j < NT; ++j) {
-        const uint2 cp = lds_u64(coff_u32 + (uint32_t)((j * 8 + 2 * t) * 4));
-        s[j][0] = lds_f32(r0a + cp.x); s[j][1] = lds_f32(r0a + cp.y);
-        s[j][2] = lds_f32(r1a + cp.x); s[j][3] = lds_f32(r1a + cp.y);
-        if (j == NT - 1) {
-          if (j * 8 + 2 * t >= n_kv) s[j][0] = s[j][2] = -1e30f;
-          if (j * 8 + 2 * t + 1 >= n_kv) s[j][1] = s[j][3] = -1e30f;
-        }
-        const __nv_bfloat16* kr = ks + (j * 8 + g) * PQ + hl * HD;
-        const uint32_t kb0 = *reinterpret_cast<const uint32_t*>(kr + 2 * t);
-        const uint32_t kb1 = *reinterpret_cast<const uint32_t*>(kr + 2 * t + 8);
-        mma16816(s[j], qa, kb0, kb1);
-      }
-      float mx0 = -INFINITY, mx1 = -INFINITY;
-#pragma unroll
-      for (int j = 0; j < NT; ++j) {
-        mx0 = fmaxf(mx0, fmaxf(s[j][0], s[j][1]));
-        mx1 = fmaxf(mx1, fmaxf(s[j][2], s[j][3]));
-      }
-      mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1));
-      mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 2));
-      mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1));
-      mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
-      const float m0s = mx0 * kLog2e, m1s = mx1 * kLog2e;
-      uint32_t pp[NT][2];
-#pragma unroll
-      for (int j = 0; j < NT; ++j) {
-        pp[j][0] = ex2_h2(fmaf(s[j][0], kLog2e, -m0s), fmaf(s[j][1], kLog2e, -m0s));
-        pp[j][1] = ex2_h2(fmaf(s[j][2], kLog2e, -m1s), fmaf(s[j][3], kLog2e, -m1s));
-      }
-      float o[2][4], ol[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-      for (int v = 0; v < 2; ++v) o[v][0] = o[v][1] = o[v][2] = o[v][3] = 0.f;
-#pragma unroll
-      for (int kk = 0; kk < KSTEPS; ++kk) {
-        uint32_t pa[4];
-        pa[0] = pp[2 * kk][0];
-        pa[1] = pp[2 * kk][1];
-        pa[2] = 2 * kk + 1 < NT ? pp[2 * kk + 1][0] : 0u;
-        pa[3] = 2 * kk + 1 < NT ? pp[2 * kk + 1][1] : 0u;
-#pragma unroll
-        for (int v = 0; v < 2; ++v) {
-          uint32_t vb0, vb1;
-          ldsm_x2_trans(vb0, vb1, vs_u32 + (uint32_t)(((kk * 16 + (lane & 15)) * PQ + hl * HD + 8 * v) * 2));
-          mma16816_f16(o[v], pa, vb0, vb1);
-        }
-        mma16816_f16(ol, pa, kOnes, kOnes);   // row sums
-      }
-      const float inv0 = 1.0f / ol[0], inv1 = 1.0f / ol[2];
-#pragma unroll
-      for (int v = 0; v < 2; ++v) {
-        const int col = hg * 64 + hl * HD + 8 * v + 2 * t;
-        *reinterpret_cast<uint32_t*>(os + row0 * PX + col) = pack2(o[v][0] * inv0, o[v][1] * inv0);
-        *reinterpret_cast<uint32_t*>(os + row1 * PX + col) = pack2(o[v][2] * inv1, o[v][3] * inv1);
-      }
-    }
-    if (dbg) t_attn += clock64() - t0;
-    // the next slice_gemm starts with a __syncthreads(): q / k / v tiles are not rewritten before every warp is past here
-  }
-  const long long t_p0 = dbg ? clock64() : 0;
-
-  // ---- output projection + window_reverse + shortcut: x[pix] += proj(o) + b, 64 output columns per weight slice --------
-  for (int js = 0; js < 4; ++js) {
-    float acc[1][2][4];
-    acc[0][0][0] = acc[0][0][1] = acc[0][0][2] = acc[0][0][3] = acc[0][1][0] = acc[0][1][1] = acc[0][1][2] = acc[0][1][3] = 0.f;
-    slice_gemm(acc, 1, os_u32, [&](int i, int r) { return mq * 16 + r; });
-#pragma unroll
-    for (int hrow = 0; hrow < 2; ++hrow) {
-      const int r = mq * 16 + g + hrow * 8;
-      const int pix = r < kTok ? pix_s[r] : -1;
-      if (pix >= 0) {
-#pragma unroll
-        for (int n = 0; n < 2; ++n) {
-          const int col = js * 64 + npair * 16 + n * 8 + 2 * t;
-          const float2 bb = __ldg(reinterpret_cast<const float2*>(p.bproj + col));
-          float2* dst = reinterpret_cast<float2*>(p.xs + (size_t)pix * C + col);
-          float2 cur = *reinterpret_cast<const float2*>(p.frames[p.q_slot] + (size_t)pix * C + col);   // shortcut = query frame
-          cur.x += acc[0][n][hrow * 2 + 0] + bb.x;
-          cur.y += acc[0][n][hrow * 2 + 1] + bb.y;
-          *dst = cur;
-        }
-      }
-    }
-  }
-  if (dbg && tid == 0) {
-    long long* o = p.dbg + (size_t)blockIdx.x * 8;
-    const long long t_end = clock64();
-    o[0] = t_end - t_begin; o[1] = t_ln; o[2] = t_gather; o[3] = t_gemm; o[4] = t_tbl; o[5] = t_attn; o[6] = t_end - t_p0;
-  }
-}
-
-template <int NT, bool kPre>
-int launch_win256(const FusedAttnParams& p, cudaStream_t s) {
-  using Cfg = WinCfg<NT, kPre>;
-  auto kern = attn_win256_kernel<NT, kPre>;
-  if (first_use_on_device((const void*)kern)) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM);
-    BDE_REQUIRE(e == cudaSuccess, "bde_window_attention_fused: smem attribute (%d bytes): %s", Cfg::SMEM, cudaGetErrorString(e));
-  }
-  FusedAttnParams q = p;
-  q.dbg = (tc::g_dbg != nullptr && (size_t)p.n_win <= tc::g_dbg_ctas) ? tc::g_dbg : nullptr;
-  const cudaError_t le = launch_pdl(kern, (unsigned)p.n_win, (unsigned)kThreadsW, (size_t)Cfg::SMEM, s, 1, q);
-  BDE_REQUIRE(le == cudaSuccess, "bde_window_attention_fused: launch: %s", cudaGetErrorString(le));
-  return check_launch("attn_win256_kernel");
 }
 
 }  // namespace
@@ -1352,7 +826,6 @@ extern "C" int bde_window_attention_fused(const float* const* frames_host, int D
   p.xs = xs;
   p.o_out = (__nv_bfloat16*)o_out;
   p.n_win = n_win; p.D = D; p.q_slot = q_slot; p.heads = heads;
-  for (int i = 0; i < 8; ++i) { p.kvpre[i] = nullptr; p.kv_ld[i] = 0; }
   p.dbg = nullptr;
   cudaStream_t s = (cudaStream_t)stream;
 #define BDE_FUSED(C_, HD_)                                       \
@@ -1361,70 +834,11 @@ extern "C" int bde_window_attention_fused(const float* const* frames_host, int D
     case 2: return launch_fused<C_, HD_, 13>(p, s);              \
     default: return launch_fused<C_, HD_, 19>(p, s);             \
   }
-  if (c == 64) {
-    // BDE2VID_ATTN64_PERSIST=1 selects the persistent form (weights / bias table resident per SM, two halves walking the
-    // windows).  Measured on B200 (tools/attn64_probe.py, us per launch, one CTA per window vs persistent): 494 windows
-    // 49.7 vs 48.3, 1976 windows 158.3 vs 158.3, 3952 windows 310.4 vs 327.7 -- the 65 KB of per-window weight / table
-    // reloads were already hidden by the second co-resident CTA, and the hardware's dynamic CTA scheduling balances the
-    // windows better than the static round-robin of the persistent form; hence off by default.
-    const char* e = getenv("BDE2VID_ATTN64_PERSIST");
-    if (e != nullptr && e[0] == '1' && n_win >= 2) {
-      switch (D) {
-        case 1: return launch_fused_pers<7>(p, s);
-        case 2: return launch_fused_pers<13>(p, s);
-        default: return launch_fused_pers<19>(p, s);
-      }
-    }
-    BDE_FUSED(64, 4)
-  }
-  if (with_proj) {   // c == 256 with the projection fused: whole-window kernel
-    // default: projections on tcgen05 (attn_tc256.cu); BDE2VID_ATTN_TC256=0 selects the mma.sync form below
-    const char* e = getenv("BDE2VID_ATTN_TC256");
-    if (!(e != nullptr && e[0] == '0') && (((uintptr_t)wqkv) & 127) == 0 && (((uintptr_t)wproj) & 127) == 0)
-      return tc::attn_win256_tc_launch(frames_host, D, q_slot, tok_map, n_win, wqkv, bqkv, bias_tbl, wproj, bproj, xs, s);
-    switch (D) {
-      case 1: return launch_win256<7, false>(p, s);
-      case 2: return launch_win256<13, false>(p, s);
-      default: return launch_win256<19, false>(p, s);
-    }
-  }
+  if (c == 64) BDE_FUSED(64, 4)
+  // c == 256 with the projection fused: whole-window kernel, projections on tcgen05 (attn_tc256.cu; it refuses weights
+  // that are not 128-byte aligned)
+  if (with_proj)
+    return tc::attn_win256_tc_launch(frames_host, D, q_slot, tok_map, n_win, wqkv, bqkv, bias_tbl, wproj, bproj, xs, s);
   BDE_FUSED(256, 16)
 #undef BDE_FUSED
-}
-
-extern "C" int bde_window_attention_fused_kvpre(const float* xq, const void* const* kv_host, const int* kv_ld, int D, int q_slot,
-                                                const int* tok_map, int n_win, int c, int heads, const void* wqkv,
-                                                const float* bqkv, const float* bias_tbl, const void* wproj, const float* bproj,
-                                                float* xs, void* stream) {
-  if (n_win == 0) return 0;
-  BDE_REQUIRE(c == 256 && heads == 16 && D >= 2 && D <= 3, "bde_window_attention_fused_kvpre: c = 256, 16 heads, D in {2, 3}");
-  BDE_REQUIRE(q_slot >= 0 && q_slot < D && xq != nullptr && kv_host != nullptr && kv_ld != nullptr && tok_map != nullptr &&
-                  wqkv != nullptr && bqkv != nullptr && bias_tbl != nullptr && wproj != nullptr && bproj != nullptr && xs != nullptr,
-              "bde_window_attention_fused_kvpre: bad arguments");
-  FusedAttnParams p;
-  for (int i = 0; i < 8; ++i) {
-    p.frames[i] = nullptr;
-    p.kvpre[i] = nullptr;
-    p.kv_ld[i] = 0;
-  }
-  p.frames[q_slot] = xq;
-  for (int d = 0; d < D; ++d) {
-    if (d == q_slot) continue;
-    p.kvpre[d] = (const __nv_bfloat16*)kv_host[d];
-    p.kv_ld[d] = kv_ld[d];
-    BDE_REQUIRE(kv_host[d] == nullptr || ((((uintptr_t)kv_host[d]) & 15) == 0 && kv_ld[d] % 8 == 0 && kv_ld[d] >= 2 * c),
-                "bde_window_attention_fused_kvpre: k / v rows must be 16-byte aligned with a pitch >= 2c");
-  }
-  p.tok_map = tok_map;
-  p.wqkv = (const __nv_bfloat16*)wqkv;
-  p.bqkv = bqkv;
-  p.tbl = bias_tbl;
-  p.wproj = (const __nv_bfloat16*)wproj;
-  p.bproj = bproj;
-  p.xs = xs;
-  p.o_out = nullptr;
-  p.dbg = nullptr;
-  p.n_win = n_win; p.D = D; p.q_slot = q_slot; p.heads = heads;
-  cudaStream_t s = (cudaStream_t)stream;
-  return D == 2 ? launch_win256<13, true>(p, s) : launch_win256<19, true>(p, s);
 }

@@ -1,9 +1,9 @@
 // Level-3 (C = 256, 16 heads of 16 channels) multi-frame window attention half with the projections on tcgen05.
 //
-// Same contract as attn_win256_kernel (attn_fused.cu): one CTA per window does window gather + LayerNorm + q / k / v
+// bde_window_attention_fused for c = 256 with the projection: one CTA per window does window gather + LayerNorm + q / k / v
 // projections + softmax(q k^T + relative-position bias) v + output projection + window_reverse + shortcut
-// (model/BDE2VID/DTransformer.py:164-207, 254-299).  What changed: the q / k / v and output projections -- 70 % of the old
-// kernel's cycles as latency-bound mma.sync slices -- are tcgen05 MMAs with the operands read once from shared memory and
+// (model/BDE2VID/DTransformer.py:164-207, 254-299).  The q / k / v and output projections -- 70 % of the cycles of the
+// earlier all-mma.sync kernel as latency-bound slices -- are tcgen05 MMAs with the operands read once from shared memory and
 // the accumulators in TMEM.  They are computed TRANSPOSED so that the weights fill the M = 128 rows of the instruction
 // exactly and the window's tokens are the N dimension (160 of 160 columns used, instead of 147 of 256 rows):
 //
@@ -41,7 +41,6 @@ struct TcAttnParams {
   const float* bproj;            // [256]
   float* xs;                     // fp32 [P, 256]
   int n_win, D, q_slot;
-  int park;                      // bring-up: workers park after the LayerNorm until the MMA warp has issued stage 16
   long long* dbg;
 };
 
@@ -557,7 +556,7 @@ attn_win256_tc_kernel(const __grid_constant__ CUtensorMap tmap_wqkv, const __gri
       worker_sync();   // q / k / v tiles and the bias table visible to every worker warp
       if (dbg) { const long long t1 = clock64(); t_conv += t1 - t0; t0 = t1; }
 
-      // ---- attention: warp = (head of the group, 16-row query tile); scores stay in registers (as attn_win256_kernel) ----
+      // ---- attention: warp = (head of the group, 16-row query tile); scores stay in registers ----------------------------
       {
         const int hl = warp >> 2, mt = warp & 3;
         const int row0 = mt * 16 + g, row1 = row0 + 8;
@@ -816,10 +815,6 @@ int attn_win256_tc_launch(const float* const* frames, int D, int q_slot, const i
   p.bproj = bproj;
   p.xs = xs;
   p.n_win = n_win; p.D = D; p.q_slot = q_slot;
-  {
-    const char* e = getenv("BDE2VID_ATTN_TC256_PARK");
-    p.park = (e != nullptr && e[0] == '1') ? 1 : 0;
-  }
   // a 2-CTA cluster per window while both CTAs of every window still fit one wave (one sequence: 35 windows -> 70 CTAs)
   int cl = 2 * n_win <= device_sm_count() ? 2 : 1;
   if (const char* e = getenv("BDE2VID_ATTN_TC256_CLUSTER")) {

@@ -207,15 +207,8 @@ class Engine:
         self.fuse_attn = os.environ.get("BDE2VID_FUSED_ATTN", "1") != "0"
         self.fuse_mlp = os.environ.get("BDE2VID_FUSED_MLP", "1") != "0"
         self.fuse_win256 = os.environ.get("BDE2VID_ATTN_WIN256", "1") != "0"
-        # the whole-window C = 256 kernel (tcgen05 projections, attn_tc256.cu) is used from this many windows up; the mma.sync
-        # form it replaced only paid off from 64 windows (one CTA per window), the tcgen05 form wins at every size measured
-        # (35 windows: 31.7 us vs 64.5 us per launch; tools/attn_tc256_probe.py)
-        self.win256_min = int(os.environ.get("BDE2VID_WIN256_MIN", "1" if os.environ.get("BDE2VID_ATTN_TC256", "1") != "0" else "64"))
-        # precomputed neighbour k | v for the level-3 attention (bde_window_attention_fused_kvpre): OFF by default.
-        # Measured on B200 (round 1): the attention kernel stays at 66 us per launch with 60 % fewer MMAs and a 5-deep
-        # weight prefetch (it is bound by barrier / shared-memory latency at 16 warps per SM, not by the projections),
-        # while the extra LayerNorm + 1x1-conv launches cost ~12 us per frame: 1982 vs 2021 frames/s.
-        self.kv_pre = os.environ.get("BDE2VID_ATTN_KVPRE", "0") != "0"
+        # the whole-window C = 256 kernel (tcgen05 projections, attn_tc256.cu) is used from this many windows up
+        self.win256_min = int(os.environ.get("BDE2VID_WIN256_MIN", "1"))
         if self.bins > VOX_CPAD:
             raise NotImplementedError("num_bins > %d" % VOX_CPAD)
         dt = self.dtype
@@ -279,8 +272,6 @@ class Engine:
                             bqkv = torch.cat([sc * (Wq @ btq + bq), Wkv @ btk + bkv], 0)
                             w, ld = _pack_linear(Wqkv, dt)
                             b["qkv"] = _Layer(w, ld, bqkv.contiguous(), 3 * C)
-                            # rows [C, 3C) = k | v: the projection of the neighbour frames, precomputable outside the chain
-                            b["kv_l"] = _Layer(w[C:], ld, bqkv[C:].contiguous(), 2 * C)
                             W1, b1 = blk.mlp.fc1.weight.detach().float(), blk.mlp.fc1.bias.detach().float()
                             g2, bt2 = blk.norm2.weight.detach().float(), blk.norm2.bias.detach().float()
                             w, ld = _pack_linear(W1 * g2[None, :], dt)
@@ -308,11 +299,6 @@ class Engine:
                                 b["red"] = (_f32(rc.weight.reshape(rc.weight.shape[0], -1)), _f32(rc.bias), n_kvf)
                         blocks.append(b)
                 self.attn.append(blocks)
-                # all blocks' k | v projections stacked: one LayerNorm-GEMM per finished frame (the "past" neighbour)
-                if blocks and all("kv_l" in b for b in blocks):
-                    w_all = torch.cat([b["kv_l"].w for b in blocks], 0).contiguous()
-                    b_all = torch.cat([b["kv_l"].bias for b in blocks], 0).contiguous()
-                    blocks[0]["kv_all"] = _Layer(w_all, blocks[0]["kv_l"].w_ld, b_all, w_all.shape[0])
             # last level with depth 0: ParseLayer + ResidualBlockNoBN x n (...V5.py:77-80, 261-282)
             self.tail = None
             if self.depths[-1] == 0:
@@ -444,7 +430,6 @@ class PairSplit:
 
 
 # kernel routes of one attention block (attention_routes; _Plan._attention_block runs them)
-KVPRE = "kvpre"        # window_attention_fused_kvpre: neighbour k | v precomputed once per frame (BDE2VID_ATTN_KVPRE=1)
 WHOLE = "whole"        # window_attention_fused, projection + scatter in the kernel
 SPLIT = "split"        # window_attention_fused to the window output, then the proj + scatter GEMM
 QKV = "qkv"            # LayerNorm-gather qkv GEMM, window_attention_mma_qkv, proj + scatter GEMM
@@ -456,12 +441,8 @@ def attention_routes(eng, l, C, nwin):
     the blocks of the fused routes run their MLP as one kernel (else as two GEMMs)."""
     blocks = eng.attn[l]
     mlp_fused = eng.fuse_mlp and ops.mlp_fused_supported(C, 4 * C)
-    if (C == 256 and eng.fuse_win256 and eng.kv_pre and nwin >= 64 and list(eng.buf) == [-1, 0, 1] and eng.q_ind == 1
-            and all(b["tbl"] is not None for b in blocks)):
-        return [KVPRE] * len(blocks), mlp_fused
-    # C = 256: the whole-window kernel (gather + LN once per window, projection + scatter fused) once there are enough
-    # windows to fill the SMs with one CTA each; below that (a single sequence has 35 level-3 windows) the per-head-group
-    # kernel's 4 CTAs per window finish sooner
+    # C = 256: the whole-window kernel (gather + LN once per window, tcgen05 projections, projection + scatter fused)
+    # from eng.win256_min windows up (by default always); the per-head-group kernel and the proj GEMM otherwise
     whole = C == 64 or (eng.fuse_win256 and nwin >= eng.win256_min)
     return [(WHOLE if whole else SPLIT) if b["tbl"] is not None else QKV if "qkv" in b else UNFUSED
             for b in blocks], mlp_fused
@@ -531,13 +512,6 @@ class _Plan:
                         d["kvr"] = E(nwin * eng.D * n_kvf, C, dtype=f32)
                 if UNFUSED in routes or not mlp_fused:
                     d.update(yn=E(P, C), hid=E(P, 4 * C))
-                if KVPRE in routes:
-                    # precomputed neighbour k | v: future frames for every block and frame, past frame ping-pong
-                    d["kv_fut"] = E(len(routes), T, P, 2 * C)
-                    d["kv_past"] = [E(P, len(routes) * 2 * C) for _ in range(2)]
-                    d["xn_all"] = E(T * P, C)          # LayerNorm'ed (no affine: folded into the weights) features, bf16
-                    d["ln_one"] = torch.ones(C, dtype=f32, device=dev)
-                    d["ln_zero"] = torch.zeros(C, dtype=f32, device=dev)
             elif l == eng.L - 1 and eng.tail is not None:
                 P = B * h * w
                 # ResidualBlockNoBN tail: running x (fp32 + operand copy) and the conv1 output
@@ -851,21 +825,13 @@ class _Plan:
         feat = d["feat"].view(T, P, C)
         feat_t = d["feat_t"].view(T, P, C)
         xs, routes = d["xs"], d["routes"]
-        pre = KVPRE in routes
-        if pre:
-            # k | v of the (pre-attention) future neighbours, all frames at once per block
-            # (one LayerNorm pass, then per block a 1x1 convolution over the [T*B, h, w, C] map on the TMA conv kernel)
-            ops.layernorm(feat.view(T * P, C), T * P, C, d["ln_one"], d["ln_zero"], d["xn_all"])
-            for i, blk in enumerate(eng.attn[l]):
-                eng.gemm(blk["kv_l"], d["xn_all"], d["kv_fut"][i].view(T * P, 2 * C), T * B, h, w, C)
-            self.launches += 1 + len(eng.attn[l])
         for t in range(T):
             # past neighbours are already post-attention (updated in place), future ones are not: quirk Q1
             frames = [feat[t + o] if 0 <= t + o < T else None for o in eng.buf]      # None = all-zero map (Q4)
             qsrc = frames[eng.q_ind]
             # the first block (plain windows: every pixel belongs to exactly one window) of the fused-projection kernels
             # reads the query frame / shortcut straight from feat[t] and writes x: no copy of feat[t] into xs
-            direct0 = qsrc is not None and routes[0] in (WHOLE, KVPRE)
+            direct0 = qsrc is not None and routes[0] == WHOLE
             if not direct0:
                 if qsrc is None:
                     xs.zero_()
@@ -879,23 +845,17 @@ class _Plan:
                 sum_args = (feat[t], feat_t[t]) if last else (None, None)
                 fr = list(frames)
                 fr[eng.q_ind] = qsrc if (direct0 and i == 0) else xs
-                sum_done = self._attention_block(route, i, blk, d, fr, t, sum_args)
+                sum_done = self._attention_block(route, i, blk, d, fr, sum_args)
             # x + merged[t], stored back in place (...V5.py:166-169), unless the last MLP kernel already did it
             if not sum_done:
                 ops.add(xs, feat[t], out_f32=feat[t], out_t=None if eng.dtype == torch.float32 else feat_t[t],
                         dtype=eng.dtype)
                 self.launches += 1
-            if pre and t + 1 < T:
-                # this frame is final: its k | v for every block of the next step (the "past" neighbour there)
-                xn_t = d["xn_all"][t * P:(t + 1) * P]      # (its pre-attention copy is not needed any more)
-                ops.layernorm(feat[t], P, C, d["ln_one"], d["ln_zero"], xn_t)
-                eng.gemm(eng.attn[l][0]["kv_all"], xn_t, d["kv_past"][t & 1], B, h, w, C)
-                self.launches += 2
             if on_frame_done is not None:
                 on_frame_done(t)
 
-    def _attention_block(self, route, i, blk, d, fr, t, sum_args):
-        """Block ``i`` at frame ``t`` along its route, in place on xs (``fr``: its input frames).  Returns True when the
+    def _attention_block(self, route, i, blk, d, fr, sum_args):
+        """Block ``i`` along its route, in place on xs (``fr``: its input frames).  Returns True when the
         block's MLP kernel also did the "x + merged" sum of ``sum_args``."""
         eng, C, nwin, ntok, D, xs = self.eng, d["C"], d["nwin"], d["ntok"], self.eng.D, d["xs"]
         P = xs.shape[0]
@@ -931,16 +891,7 @@ class _Plan:
             eng.gemm(blk["fc2"], d["hid"], xs, 1, P, 1, 4 * C, out_f32=True, residual=xs)
             self.launches += 7
             return False
-        if route == KVPRE:
-            kv = [None] * D
-            if t >= 1:
-                kv[0] = d["kv_past"][(t - 1) & 1][:, i * 2 * C:(i + 1) * 2 * C]
-            if t + 1 < self.T:
-                kv[2] = d["kv_fut"][i, t + 1]
-            ops.window_attention_fused_kvpre(fr[eng.q_ind], kv, eng.q_ind, tm.view(-1), nwin, C, eng.heads, blk["qkv"].w,
-                                             blk["qkv"].bias, blk["tbl"], blk["proj"].w, blk["proj"].bias, xs)
-            self.launches += 1
-        elif route == WHOLE:
+        if route == WHOLE:
             ops.window_attention_fused(fr, eng.q_ind, tm.view(-1), nwin, C, eng.heads, blk["qkv"].w, blk["qkv"].bias,
                                        blk["tbl"], blk["proj"].w, blk["proj"].bias, xs=xs)
             self.launches += 1

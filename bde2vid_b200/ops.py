@@ -277,21 +277,6 @@ def window_attention_fused(frames, q_slot, tok_map, n_win, c, heads, wqkv, bqkv,
           "bde_window_attention_fused")
 
 
-def window_attention_fused_kvpre(xq, kv, q_slot, tok_map, n_win, c, heads, wqkv, bqkv, bias_tbl, wproj, bproj, xs):
-    """Whole-window attention half for c = 256 with precomputed neighbour k / v.  ``kv``: list of length D with, per
-    neighbour slot, None (zero frame) or a bf16 2-D tensor view [P, >= 2c] (row pitch = stride(0)); kv[q_slot] ignored."""
-    lib = _lib.require_device()
-    D = len(kv)
-    ptrs = (C.c_void_p * D)(*[None if (t is None or d == q_slot) else t.data_ptr() for d, t in enumerate(kv)])
-    lds = (C.c_int * D)(*[0 if (t is None or d == q_slot) else t.stride(0) for d, t in enumerate(kv)])
-    for d, t in enumerate(kv):
-        if t is not None and d != q_slot:
-            assert t.dtype == torch.bfloat16 and t.stride(1) == 1 and t.shape[1] >= 2 * c
-    check(lib.bde_window_attention_fused_kvpre(ptr(xq), ptrs, lds, D, q_slot, ptr(tok_map), n_win, c, heads, ptr(wqkv), ptr(bqkv),
-                                               ptr(bias_tbl), ptr(wproj), ptr(bproj), ptr(xs), stream_ptr()),
-          "bde_window_attention_fused_kvpre")
-
-
 def mlp_fused_supported(c, hidden):
     return _lib.load().bde_mlp_fused_supported(c, hidden) == 1
 

@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define BDE_ABI_VERSION 2
+#define BDE_ABI_VERSION 3
 
 /* element types of activation / weight buffers */
 enum { BDE_F32 = 0, BDE_BF16 = 1 };
@@ -304,23 +304,15 @@ int bde_window_attention_mma_qkv(const void* qkv, const float* bias_padded, int 
  *   c == 64 : wproj bf16 [c, c], bproj float32 [c]; xs float32 [P, c] (= frames_host[q_slot]) receives
  *             xs[pix] += proj(attn)[token] + bproj for every covered pixel (window_reverse + crop + shortcut)
  *   c == 256: o_out bf16 [n_win * 49, c] receives the attention output (heads concatenated); the caller
- *             runs proj as a bde_gemm with BDE_EPI_SCATTER
+ *             runs proj as a bde_gemm with BDE_EPI_SCATTER.  With wproj, bproj and xs given instead, the
+ *             projection is fused as for c == 64 (one whole-window tcgen05 kernel); wqkv and wproj must then
+ *             be 128-byte aligned (the call fails otherwise)
  * Supported: 7x7 windows, D <= 3, (c, heads) with c in {64, 256} and head_dim = c / 64 * 4 (4 or 16);
  * bde_window_attention_fused_supported returns 1 for a supported shape. */
 int bde_window_attention_fused_supported(int c, int heads, int n_tok, int D);
 int bde_window_attention_fused(const float* const* frames_host, int D, int q_slot, const int* tok_map, int n_win,
                                int c, int heads, const void* wqkv, const float* bqkv, const float* bias_tbl,
                                const void* wproj, const float* bproj, float* xs, void* o_out, void* stream);
-
-/* Whole-window form for c = 256 with the k / v rows of the D - 1 neighbour frames precomputed (they do not depend on the
- * running x, DTransformer.py:376-389: only frames[q_ind] changes inside the block stack): LayerNorm-GEMM launches
- * (bde_gemm, ln_mode = 1, weights = rows [c, 3c) of wqkv) write bf16 [P, >= 2c] rows = [k | v]; this kernel gathers them
- * per window, normalises + projects only the 49 query-frame tokens, and fuses attention, projection, window_reverse and
- * the shortcut into xs.  kv_host[d] = NULL means an all-zero neighbour frame; kv_host[q_slot] is ignored.
- *   xq: float32 [P, c] query frame (may alias xs)   kv_ld[d]: row pitch of kv_host[d] in elements */
-int bde_window_attention_fused_kvpre(const float* xq, const void* const* kv_host, const int* kv_ld, int D, int q_slot,
-                                     const int* tok_map, int n_win, int c, int heads, const void* wqkv, const float* bqkv,
-                                     const float* bias_tbl, const void* wproj, const float* bproj, float* xs, void* stream);
 
 /* Fused MLP half of a SwinTransformerBlock3D (DTransformer.py:279-283,302-304), in place on the fp32
  * residual stream:  x[m, :] += fc2(GELU(fc1(LayerNorm(x[m, :]))))   for x float32 [rows, c].

@@ -23,7 +23,7 @@ def test_library_exports_every_declared_symbol(lib_built):
     for s in syms:
         assert hasattr(lib, s), "libbde2vid_sm100.so does not export %s" % s
     lib.bde_abi_version.restype = ctypes.c_int
-    assert lib.bde_abi_version() == 2
+    assert lib.bde_abi_version() == 3
     lib.bde_last_error.restype = ctypes.c_char_p
     assert lib.bde_last_error() is not None
 

@@ -1,5 +1,5 @@
-"""Kernel-level float64 references for the fused window-attention kernels (bde_window_attention_fused,
-bde_window_attention_fused_kvpre: attn_fused.cu, attn_tc256.cu) and the fused transformer MLPs (bde_mlp_fused,
+"""Kernel-level float64 references for the fused window-attention kernels (bde_window_attention_fused:
+attn_fused.cu, attn_tc256.cu) and the fused transformer MLPs (bde_mlp_fused,
 bde_mlp_fused_sum: mlp_fused.cu), one case per kernel instance, in the call forms the engine makes.
 
 The references restate DTransformer.py:183-207 (WindowAttention3D) and 279-306 (the block's shortcut and MLP) in plain
@@ -51,7 +51,7 @@ a gate of ulp + e, tight by construction), 0.17 on the fp32 updates of the C = 6
 kernels, 0.18 / 0.08 on the C = 64 / C = 256 MLPs.
 
 Every case prints its largest err / gate and asserts, with torch.profiler, which kernel instance served it; the test ids
-name the instances (all 24 of profiles/sass/{attn_fused,attn_tc256,mlp_fused}.kernels.txt).  Each family also checks that
+name the instances (all 16 of profiles/sass/{attn_fused,attn_tc256,mlp_fused}.kernels.txt).  Each family also checks that
 a plausibly wrong reference fails the same gate.  (tanh-GELU is not among them: it differs from erf-GELU by at most
 1.8e-4 |h|, inside the 2.4e-4 |h| that tanh.approx alone is allowed, so no sound gate can separate the two.)
 
@@ -129,11 +129,10 @@ def win_tokens(f, tm):
     return f[tm.clamp(min=0)] * (tm >= 0).unsqueeze(-1).to(F64)
 
 
-def attn_ref(frames, q_slot, tm, wqkv, bqkv, tbl, wproj, bproj, heads, kvpre=None, exact=False, ln_eps=LN_EPS,
-             wrong=None, chunk=None):
+def attn_ref(frames, q_slot, tm, wqkv, bqkv, tbl, wproj, bproj, heads, exact=False, ln_eps=LN_EPS, wrong=None,
+             chunk=None):
     """Attention half in float64 with mirrored stores.  frames: D float64 [P, C] maps or None; tm: long [nwin, 49];
-    wqkv / wproj: float64 values of the bf16 weights; kvpre: per slot None or float64 [P, 2C] k | v rows (bf16 values;
-    the query slot is ignored).  wrong: None, "mirror_tbl", "softmax_per_frame" or "drop_zero_keys".
+    wqkv / wproj: float64 values of the bf16 weights.  wrong: None, "mirror_tbl", "softmax_per_frame" or "drop_zero_keys".
     Returns (o, d_o [nwin * 49, C], y, e_y [nwin * 49, C]); y and e_y are None without wproj."""
     D = len(frames)
     C = wqkv.shape[1]
@@ -154,17 +153,8 @@ def attn_ref(frames, q_slot, tm, wqkv, bqkv, tbl, wproj, bproj, heads, kvpre=Non
         nw = t.shape[0]
         ks, dks, vs, dvs, valid = [], [], [], [], []
         for d in range(D):
-            src = win_tokens(frames[d], t) if (kvpre is None or d == q_slot) else None
-            valid.append((t >= 0) & (frames[d] is not None if kvpre is None or d == q_slot else kvpre[d] is not None))
-            if kvpre is not None and d != q_slot:
-                # precomputed neighbour k | v as given (bf16); zero tokens take the bias rounded to bf16
-                kvz = torch.cat([rnd(bk, BF), rnd(bv, BF)]).expand(nw, 49, 2 * C)
-                kv = kvz if kvpre[d] is None else torch.where((t >= 0).unsqueeze(-1), kvpre[d][t.clamp(min=0)], kvz)
-                ks.append(kv[..., :C])
-                dks.append(torch.zeros_like(kv[..., :C]))
-                vs.append(rnd(kv[..., C:], F16))
-                dvs.append(torch.zeros_like(kv[..., :C]))
-                continue
+            src = win_tokens(frames[d], t)
+            valid.append((t >= 0) & (frames[d] is not None))
             if src is None:
                 src = torch.zeros(nw, 49, C, dtype=F64, device=dev)
             xhat, ex = ln_ref(src, ln_eps)
@@ -245,13 +235,13 @@ def mlp_ref(x, w1, b1, w2, b2, exact=False, ln_eps=LN_EPS, gelu=F.gelu):
 # ---------------------------------------------------------------------------------------------------------------------
 # kernel instances
 # ---------------------------------------------------------------------------------------------------------------------
-_KERNEL = re.compile(r"(attn_fused_kernel|attn_win256_tc_kernel|attn_win256_kernel|mlp_fused256_kernel|mlp_fused_kernel)"
+_KERNEL = re.compile(r"(attn_fused_kernel|attn_win256_tc_kernel|mlp_fused256_kernel|mlp_fused_kernel)"
                      r"(?:<([^<>]*)>|I((?:L[ib]\d+E)+)E)?")
 
 
 def instances(names):
     """Instance strings (``base<arg, ...>`` as in profiles/sass/*.kernels.txt) of the fused kernels among ``names``,
-    from demangled (``attn_fused_kernel<64, 4, 7, false>``) or mangled (``attn_fused_kernelILi64ELi4ELi7ELb0EE``) names."""
+    from demangled (``attn_fused_kernel<64, 4, 7>``) or mangled (``attn_fused_kernelILi64ELi4ELi7EE``) names."""
     out = set()
     for n in names:
         for m in _KERNEL.finditer(n):
@@ -360,12 +350,9 @@ def run_update(S, frames, q_slot, tm, inst, direct, name, wrongs=(), **kw):
     return xs
 
 
-ATTN64 = ["attn_fused_kernel<64, 4, %d, false>" % nt for nt in (7, 13, 19)]
-ATTN64_PERS = ["attn_fused_kernel<64, 4, %d, true>" % nt for nt in (7, 13, 19)]
+ATTN64 = ["attn_fused_kernel<64, 4, %d>" % nt for nt in (7, 13, 19)]
 TC256 = ["attn_win256_tc_kernel<%d, %d>" % (nt, cl) for nt in (7, 13, 19) for cl in (1, 2)]
-WIN256 = ["attn_win256_kernel<%d, false>" % nt for nt in (7, 13, 19)]
-KVPRE = ["attn_win256_kernel<%d, true>" % nt for nt in (13, 19)]
-HG256 = ["attn_fused_kernel<256, 16, %d, false>" % nt for nt in (7, 13, 19)]
+HG256 = ["attn_fused_kernel<256, 16, %d>" % nt for nt in (7, 13, 19)]
 MLP64 = "mlp_fused_kernel"
 MLP256 = ["mlp_fused256_kernel<%d>" % cl for cl in (1, 2, 4)]
 NT_D = {7: 1, 13: 2, 19: 3}
@@ -381,7 +368,7 @@ def nt_of(inst):
 @gpu
 @pytest.mark.parametrize("inst", ATTN64)
 def test_attn64(inst):
-    """attn_fused_kernel<64, 4, NT, false> on the model's level-1 map (132 x 176: 494 ragged windows): q_slot at every
+    """attn_fused_kernel<64, 4, NT> on the model's level-1 map (132 x 176: 494 ragged windows): q_slot at every
     position, a None frame in each non-query slot, plain and dilated maps, in-place and direct forms, bias tables at
     scale 0.02 and 1.0."""
     D = NT_D[nt_of(inst)]
@@ -405,38 +392,6 @@ def test_attn64(inst):
                 run_update(S, frames, q_slot, tms[dil], inst, direct=not dil,
                            name="%s q%d zero%s dil%d tbl%d" % (inst, q_slot, zero, dil, run % 2), wrongs=wrongs)
             run += 1
-
-
-@gpu
-@pytest.mark.parametrize("inst", ATTN64_PERS)
-def test_attn64_persistent(inst, monkeypatch):
-    """attn_fused_kernel<64, 4, NT, true> (BDE2VID_ATTN64_PERSIST=1) on two level-1 maps (988 windows: each of the
-    2 x SMs halves walks several) sliced to an odd (987) and an even (988) window count, in place: bit-identical to the
-    one-window-per-CTA form, within the gate of the reference, and the pixels of the sliced-off window bit-unchanged.
-    n_win = 1 falls back to the per-window kernel."""
-    NT = nt_of(inst)
-    D = NT_D[NT]
-    q_slot = D // 2
-    H, W = 132, 176
-    S = AttnSetup(64, D, 2 * H * W, seed=7 + NT, tbl_scale=1.0)
-    frames = list(S.frames)
-    if D > 1:
-        frames[(q_slot + 1) % D] = None
-    full = tmap(2, H, W, True)
-    assert full.shape[0] == 988
-    for n in (987, 988):
-        tm = full[:n].contiguous()
-        monkeypatch.setenv("BDE2VID_ATTN64_PERSIST", "1")
-        xp = run_update(S, frames, q_slot, tm, inst, direct=False, name="%s n_win %d" % (inst, n))
-        monkeypatch.setenv("BDE2VID_ATTN64_PERSIST", "0")
-        xs = frames[q_slot].clone()
-        fr = list(frames)
-        fr[q_slot] = xs
-        run_routed(lambda: S.launch(fr, q_slot, tm, xs=xs), "attn_fused_kernel<64, 4, %d, false>" % NT)
-        assert torch.equal(xp, xs), "persistent and one-window-per-CTA forms differ"
-    monkeypatch.setenv("BDE2VID_ATTN64_PERSIST", "1")
-    run_update(S, frames, q_slot, full[:1].contiguous(), "attn_fused_kernel<64, 4, %d, false>" % NT, direct=False,
-               name="%s n_win 1 -> per-window kernel" % inst)
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -491,75 +446,9 @@ def test_attn256_tc(inst, monkeypatch):
 
 
 @gpu
-@pytest.mark.parametrize("inst", WIN256)
-def test_attn256_mma(inst, monkeypatch):
-    """attn_win256_kernel<NT, false> (BDE2VID_ATTN_TC256=0), 33 x 44 plain (direct) and dilated (in place)."""
-    monkeypatch.setenv("BDE2VID_ATTN_TC256", "0")
-    NT = nt_of(inst)
-    D = NT_D[NT]
-    q_slot = D - 1
-    H, W = 33, 44
-    S = AttnSetup(256, D, 2 * H * W, seed=400 + NT, tbl_scale=1.0)
-    frames = list(S.frames)
-    wr = ("mirror_tbl", "neighbour_shortcut") if D > 1 else ("drop_zero_keys",)
-    run_update(S, frames, q_slot, tmap(2, H, W, False), inst, direct=True, name="%s plain direct" % inst, wrongs=wr)
-    if D > 1:
-        frames[0] = None
-    run_update(S, frames, q_slot, tmap(2, H, W, True), inst, direct=False, name="%s dilated in place" % inst)
-
-
-@gpu
-@pytest.mark.parametrize("inst", KVPRE)
-def test_attn256_kvpre(inst):
-    """attn_win256_kernel<NT, true>: precomputed neighbour k | v rows (bf16) at pitch 2C and at the wider pitch of the
-    engine's kv_past slice (block 1 of 3), one None neighbour, q_slot in {0, 1, D - 1}, in place and direct."""
-    from bde2vid_b200 import ops
-    NT = nt_of(inst)
-    D = NT_D[NT]
-    C = 256
-    H, W = 33, 44
-    P = 2 * H * W
-    S = AttnSetup(C, D, P, seed=500 + NT, tbl_scale=1.0)
-    W64 = S.wqkv[C:].to(F64)
-    kvs = []
-    for d in range(D):      # k | v of every frame as the engine precomputes them: LayerNorm + rows [C, 3C), bf16
-        kv = (ln_ref(S.frames[d].to(F64))[0].to(BF).to(F64) @ W64.t() + S.bqkv[C:].to(F64)).to(BF)
-        wide = torch.zeros(P, 6 * C, dtype=BF, device=DEV)
-        wide[:, 2 * C:4 * C] = kv
-        kvs.append((kv.contiguous(), wide[:, 2 * C:4 * C]))
-    for i, q_slot in enumerate(sorted({0, 1, D - 1})):
-        for dil in (False, True):
-            tm = tmap(2, H, W, dil)
-            kv = [None if d == q_slot else kvs[d][(i + int(dil)) % 2] for d in range(D)]
-            zero = [d for d in range(D) if d != q_slot][int(dil) % (D - 1)]
-            if dil:
-                kv[zero] = None
-            direct = not dil
-            q = S.frames[q_slot]
-            q0 = q.clone()
-            xs = torch.full_like(q, float("nan")) if direct else q.clone()
-            xq = q if direct else xs
-            run_routed(lambda: ops.window_attention_fused_kvpre(xq, kv, q_slot, tm.view(-1), tm.shape[0], C, 16, S.wqkv,
-                                                                S.bqkv, S.tbl, S.wproj, S.bproj, xs), inst)
-            assert torch.equal(q, q0)
-            kv64 = [None if t is None else t.to(F64) for t in kv]
-            frames64 = [q0 if d == q_slot else None for d in range(D)]
-            _, _, y, e_y = S.ref(frames64, q_slot, tm, kvpre=kv64)
-            before = torch.full_like(q0, float("nan")).to(F64) if direct else q0.to(F64)
-            ref, gate = scatter_update(before, q0.to(F64), tm.long(), y, e_y)
-            name = "%s q%d dil%d pitch %d" % (inst, q_slot, dil, kv[(q_slot + 1) % D].stride(0) if kv[(q_slot + 1) % D] is not None else 0)
-            if dil:
-                # the bias table of the mirrored frame slot
-                _, _, yw, _ = S.ref(frames64, q_slot, tm, kvpre=kv64, wrong="mirror_tbl")
-                wref, _ = scatter_update(before, q0.to(F64), tm.long(), yw, e_y)
-                assert gate_ratio(xs, wref, gate) > 1.0, name
-            check(name, xs, ref, gate)
-
-
-@gpu
 @pytest.mark.parametrize("inst", HG256)
 def test_attn256_head_groups(inst):
-    """attn_fused_kernel<256, 16, NT, false>: the per-head-group form that writes the bf16 attention output o_out
+    """attn_fused_kernel<256, 16, NT>: the per-head-group form that writes the bf16 attention output o_out
     (the projection then runs as a GEMM), gated on the bf16 o store.  The token map has 35 plain windows of the 33 x 44
     map plus three windows that are entirely padding."""
     NT = nt_of(inst)
@@ -586,7 +475,8 @@ def test_attn256_head_groups(inst):
 
 @gpu
 def test_attn_refused_calls():
-    """A None query frame with the projection, and an unsupported (c, heads, D), are refused."""
+    """A None query frame with the projection, an unsupported (c, heads, D), and c = 256 with the projection and wqkv
+    16-byte but not 128-byte aligned, are refused."""
     from bde2vid_b200 import ops
     S = AttnSetup(64, 3, 14 * 14, seed=1, tbl_scale=0.02)
     tm = tmap(1, 14, 14, False)
@@ -598,6 +488,16 @@ def test_attn_refused_calls():
                                    xs=xs)
     with pytest.raises(RuntimeError):
         ops.window_attention_fused(S.frames + [S.frames[0]], 1, tm.view(-1), tm.shape[0], 64, 16, S.wqkv, S.bqkv, S.tbl,
+                                   S.wproj, S.bproj, xs=xs)
+    assert torch.equal(xs, S.frames[1])
+    S = AttnSetup(256, 3, 14 * 14, seed=2, tbl_scale=0.02)
+    buf = torch.empty(S.wqkv.numel() + 32, dtype=BF, device=DEV)
+    wqkv = buf[32:].view_as(S.wqkv)          # 64 bytes past a 128-byte aligned allocation
+    wqkv.copy_(S.wqkv)
+    assert wqkv.data_ptr() % 16 == 0 and wqkv.data_ptr() % 128 == 64
+    xs = S.frames[1].clone()
+    with pytest.raises(RuntimeError):
+        ops.window_attention_fused([S.frames[0], xs, S.frames[2]], 1, tm.view(-1), tm.shape[0], 256, 16, wqkv, S.bqkv, S.tbl,
                                    S.wproj, S.bproj, xs=xs)
     assert torch.equal(xs, S.frames[1])
 
@@ -779,12 +679,10 @@ def test_flip(dtype):
 
 # kernel names as torch.profiler reported them on a B200
 _PROFILED_NAMES = {
-    "void bde::(anonymous namespace)::attn_fused_kernel<64, 4, 13, true>(bde::(anonymous namespace)::FusedAttnParams)":
-        "attn_fused_kernel<64, 4, 13, true>",
-    "void bde::(anonymous namespace)::attn_fused_kernel<256, 16, 19, false>(bde::(anonymous namespace)::FusedAttnParams)":
-        "attn_fused_kernel<256, 16, 19, false>",
-    "void bde::(anonymous namespace)::attn_win256_kernel<13, true>(bde::(anonymous namespace)::FusedAttnParams)":
-        "attn_win256_kernel<13, true>",
+    "void bde::(anonymous namespace)::attn_fused_kernel<64, 4, 13>(bde::(anonymous namespace)::FusedAttnParams)":
+        "attn_fused_kernel<64, 4, 13>",
+    "void bde::(anonymous namespace)::attn_fused_kernel<256, 16, 19>(bde::(anonymous namespace)::FusedAttnParams)":
+        "attn_fused_kernel<256, 16, 19>",
     "void bde::tc::(anonymous namespace)::attn_win256_tc_kernel<19, 1>(CUtensorMap_st, CUtensorMap_st, "
     "bde::tc::(anonymous namespace)::TcAttnParams)": "attn_win256_tc_kernel<19, 1>",
     "void bde::tc::mlp_fused256_kernel<2>(CUtensorMap_st, CUtensorMap_st, bde::tc::Mlp3Params)": "mlp_fused256_kernel<2>",
@@ -795,16 +693,16 @@ _PROFILED_NAMES = {
 def test_instance_parser():
     """The parser reads the template arguments of the fused kernels in the demangled and the mangled form."""
     dem = {
-        "void bde::(anonymous namespace)::attn_fused_kernel<64, 4, 19, true>(bde::(anonymous namespace)::FusedAttnParams)":
-            "attn_fused_kernel<64, 4, 19, true>",
+        "void bde::(anonymous namespace)::attn_fused_kernel<64, 4, 19>(bde::(anonymous namespace)::FusedAttnParams)":
+            "attn_fused_kernel<64, 4, 19>",
         "void bde::tc::attn_win256_tc_kernel<13, 2>(CUtensorMap_st, CUtensorMap_st, bde::tc::TcAttnParams)":
             "attn_win256_tc_kernel<13, 2>",
     }
     man = {   # symbol names of the sm_100a build (cuobjdump -sass)
-        "_ZN3bde46_GLOBAL__N__b80b0db7_13_attn_fused_cu_44e2f06b17attn_fused_kernelILi256ELi16ELi7ELb0EEEvNS0_15FusedAttnParamsE":
-            "attn_fused_kernel<256, 16, 7, false>",
-        "_ZN3bde46_GLOBAL__N__b80b0db7_13_attn_fused_cu_44e2f06b18attn_win256_kernelILi19ELb1EEEvNS0_15FusedAttnParamsE":
-            "attn_win256_kernel<19, true>",
+        "_ZN3bde46_GLOBAL__N__b80b0db7_13_attn_fused_cu_44e2f06b17attn_fused_kernelILi256ELi16ELi7EEEvNS0_15FusedAttnParamsE":
+            "attn_fused_kernel<256, 16, 7>",
+        "_ZN3bde46_GLOBAL__N__b80b0db7_13_attn_fused_cu_44e2f06b17attn_fused_kernelILi64ELi4ELi19EEEvNS0_15FusedAttnParamsE":
+            "attn_fused_kernel<64, 4, 19>",
         "_ZN3bde2tc46_GLOBAL__N__1f88433e_13_attn_tc256_cu_87ba617621attn_win256_tc_kernelILi7ELi2EEEv14CUtensorMap_stS3_NS1_12TcAttnParamsE":
             "attn_win256_tc_kernel<7, 2>",
         "_ZN3bde2tc19mlp_fused256_kernelILi4EEEv14CUtensorMap_stS2_NS0_10Mlp3ParamsE": "mlp_fused256_kernel<4>",
@@ -825,5 +723,5 @@ def test_instance_ids_cover_the_build():
             for line in fh:
                 if not line.startswith("#") and line.strip():
                     listed |= instances([line.split("  ")[0]])
-    ours = set(ATTN64 + ATTN64_PERS + TC256 + WIN256 + KVPRE + HG256 + [MLP64] + MLP256)
-    assert len(listed) == 24 and listed == ours, (sorted(listed ^ ours))
+    ours = set(ATTN64 + TC256 + HG256 + [MLP64] + MLP256)
+    assert len(listed) == 16 and listed == ours, (sorted(listed ^ ours))

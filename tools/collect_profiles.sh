@@ -17,6 +17,5 @@ cp $S/voxel_traffic.csv $D/${R}_ncu_voxel_traffic.csv
 [ -s $S/voxel_probe.log ] && cp $S/voxel_probe.log $D/${R}_voxel_probe.txt
 [ -s $S/attn_phase_probe.log ] && cp $S/attn_phase_probe.log $D/${R}_attn_phase_cycles.txt
 [ -s $S/mlp_probe.log ] && cp $S/mlp_probe.log $D/${R}_mlp_probe.txt
-[ -s $S/attn_tc256_probe.log ] && cp $S/attn_tc256_probe.log $D/${R}_attn_tc256_probe.txt
 [ -s gpurun_out/bench_2gpu.json ] && [ gpurun_out/bench_2gpu.json -nt $D/r01_bench_2gpu_torchrun.json ] && cp gpurun_out/bench_2gpu.json $D/${R}_bench_2gpu_torchrun.json
 ls -la $D | grep $R

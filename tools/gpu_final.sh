@@ -15,7 +15,6 @@ done
 timeout 300 python tools/voxel_probe.py > $O/voxel_probe.log 2>&1; echo "voxel probe exit $?"
 timeout 300 python tools/attn_phase_probe.py > $O/attn_phase_probe.log 2>&1; echo "attn phase probe exit $?"
 timeout 300 python tools/mlp_probe.py > $O/mlp_probe.log 2>&1; echo "mlp probe exit $?"
-timeout 300 python tools/attn_tc256_probe.py > $O/attn_tc256_probe.log 2>&1; echo "tc256 probe exit $?"
 fi
 CMD="python bench.py --windows 6 --steps 1 --warmup 3 --concurrent 1 --batch 8 --no-cpu-baseline --no-kernel-timing --no-single"
 timeout 600 $CMD > $O/plain.log 2>&1 && \
