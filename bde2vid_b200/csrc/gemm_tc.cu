@@ -44,13 +44,13 @@ __global__ void __launch_bounds__(kThreads, kMinCtas<BN, kDeep, kLn>) gemm_tc_ke
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t smem_a = smem_base;                       // S x [128 x 128B]
   const uint32_t smem_b = smem_base + S * Cfg::kABytes;    // S x [BN x 128B]
-  const uint32_t bar_base = smem_base + S * Cfg::kStageBytes;
+  const uint32_t bar_base = smem_base + Cfg::kOperandBytes;   // after the stages and the epilogue's staging
   const uint32_t bar_full = bar_base;                      // S x 8B
   const uint32_t bar_empty = bar_base + 8 * S;             // S x 8B
   const uint32_t bar_acc = bar_base + 16 * S;              // 8B
   const uint32_t tmem_slot = bar_base + 16 * S + 8;        // 4B
   uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));  // generic pointer to smem_base
-  float* bias_s = reinterpret_cast<float*>(smem_gen + S * Cfg::kStageBytes + 256);  // BN floats
+  float* bias_s = reinterpret_cast<float*>(smem_gen + Cfg::kOperandBytes + 256);  // BN floats
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int m_tile = blockIdx.x, n0 = blockIdx.y * BN;
@@ -258,6 +258,7 @@ __global__ void __launch_bounds__(kThreads, kMinCtas<BN, kDeep, kLn>) gemm_tc_ke
     // accumulator is complete) and then works on quads: lane -> (row 4*it + lane/8, columns 4*(lane%8)..+3),
     // i.e. 8 lanes cover 128 contiguous bytes of one output row.
     constexpr int kPitch = 36;  // floats; 16-byte aligned rows, conflict-free for both access patterns
+    static_assert(kNumProducerWarps * 32 * kPitch * 4 <= Cfg::kEpiBytes, "epilogue staging outgrows TileCfg::kEpiBytes");
     float* stg = reinterpret_cast<float*>(smem_gen) + warp * (32 * kPitch);
     const int rq = lane >> 3, cq = (lane & 7) * 4;
     int m_it[8];            // output row index of (4*it + rq), -1 if outside the problem

@@ -246,7 +246,11 @@ struct TileCfg {
   static constexpr int kABytes = BM * BK * 2;
   static constexpr int kBBytes = BN * BK * 2;
   static constexpr int kStageBytes = kABytes + kBBytes;
-  static constexpr int kSmemBytes = kStages * kStageBytes + 1024 /*align slack*/ + 256 /*barriers*/ + BN * 4 /*bias*/;
+  // the epilogue transposes its accumulator chunks in the operand region (8 producer warps x 32 rows x 36 floats) once the
+  // main loop is done; a one-stage LayerNorm tile with BN <= 128 has fewer operand bytes than that
+  static constexpr int kEpiBytes = kNumProducerWarps * 32 * 36 * 4;
+  static constexpr int kOperandBytes = kStages * kStageBytes > kEpiBytes ? kStages * kStageBytes : kEpiBytes;
+  static constexpr int kSmemBytes = kOperandBytes + 1024 /*align slack*/ + 256 /*barriers*/ + BN * 4 /*bias*/;
   static constexpr int kTmemCols = BN <= 32 ? 32 : (BN <= 64 ? 64 : (BN <= 128 ? 128 : 256));
 };
 
