@@ -63,6 +63,7 @@ EXPORTS = {
                           C.c_void_p]),
     "bde_upsample2x_sum": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_float] + [C.c_int] * 4
                            + [C.c_void_p, C.c_int, C.c_void_p]),
+    "bde_shuffle2x_sum": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int] * 4 + [C.c_void_p, C.c_int, C.c_void_p]),
     "bde_pred_sigmoid": (C.c_int, [C.c_void_p] * 5 + [C.c_int, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "bde_window_reduce": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

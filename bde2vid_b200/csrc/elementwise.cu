@@ -148,6 +148,54 @@ __global__ void __launch_bounds__(256) upsample2x_sum_block_kernel(const TS* __r
 }
 
 // ---------------------------------------------------------------------------------------------
+// Pixel shuffle of a stride-2 transposed convolution run as four phase convolutions on the low-resolution map
+// (TransposedConvLayer, model/e2vid/submodules.py), plus the skip that feeds the next decoder (skip_sum, unet.py):
+//   dst[b, 2i+py, 2j+px, :] = g[b, i, j, (2py+px)*c : (2py+px+1)*c]  (+ skip[b, 2i+py, 2j+px, :])
+// Thread = one 16-byte vector of a destination row, so every row is stored coalesced; blockIdx.y walks the rows.
+// The bf16 sum is formed in fp32 and rounded once, as torch's bf16 add does.
+// ---------------------------------------------------------------------------------------------
+template <typename T>
+__device__ __forceinline__ uint4 add16(uint4 a, uint4 b);
+template <>
+__device__ __forceinline__ uint4 add16<float>(uint4 a, uint4 b) {
+  const float4 x = *reinterpret_cast<const float4*>(&a), y = *reinterpret_cast<const float4*>(&b);
+  const float4 s = make_float4(x.x + y.x, x.y + y.y, x.z + y.z, x.w + y.w);
+  return *reinterpret_cast<const uint4*>(&s);
+}
+template <>
+__device__ __forceinline__ uint4 add16<__nv_bfloat16>(uint4 a, uint4 b) {
+  const uint32_t x[4] = {a.x, a.y, a.z, a.w}, y[4] = {b.x, b.y, b.z, b.w};
+  uint32_t r[4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const float2 p = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&x[i]));
+    const float2 q = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&y[i]));
+    const __nv_bfloat162 s = __floats2bfloat162_rn(p.x + q.x, p.y + q.y);
+    r[i] = *reinterpret_cast<const uint32_t*>(&s);
+  }
+  return make_uint4(r[0], r[1], r[2], r[3]);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(256) shuffle2x_sum_kernel(const T* __restrict__ g, const T* __restrict__ skip, int h, int w,
+                                                            int cv, int rows, T* __restrict__ dst) {
+  constexpr int V = 16 / sizeof(T);                          // elements per vector
+  const int idx = blockIdx.x * blockDim.x + threadIdx.x;     // over the 2w * cv vectors of one destination row
+  if (idx >= 2 * w * cv) return;
+  const int ox = idx / cv, q = idx - ox * cv;
+  const int c = cv * V;
+  for (int r = blockIdx.y; r < rows; r += gridDim.y) {       // r = img * 2h + oy
+    const int img = r / (2 * h), oy = r - img * 2 * h;
+    const size_t src = (((size_t)img * h + (oy >> 1)) * w + (ox >> 1)) * (size_t)(4 * c) +
+                       (size_t)(((oy & 1) * 2 + (ox & 1)) * c + q * V);
+    const size_t o = (size_t)r * (size_t)(2 * w) * c + (size_t)idx * V;
+    uint4 v = __ldg(reinterpret_cast<const uint4*>(g + src));
+    if (skip != nullptr) v = add16<T>(v, __ldg(reinterpret_cast<const uint4*>(skip + o)));
+    *reinterpret_cast<uint4*>(dst + o) = v;
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
 // img = sigmoid(bias + wt . (x + head))   (predI 1x1 conv + Sigmoid, ...V5.py:195-197)
 // one thread per pixel; c <= 256, multiple of 4
 // ---------------------------------------------------------------------------------------------
@@ -433,6 +481,28 @@ extern "C" int bde_upsample2x_sum(const void* skip, int skip_f32, const void* x,
   if (n_img == 0) return 0;
   if (dtype == BDE_F32) return launch_upsample<float>(skip, 1, x, 1, x_scale, n_img, h, w, c, dst, s);
   return launch_upsample<__nv_bfloat16>(skip, skip_f32, x, x_f32, x_scale, n_img, h, w, c, dst, s);
+}
+
+extern "C" int bde_shuffle2x_sum(const void* g, const void* skip, int n_img, int h, int w, int c, void* dst, int dtype,
+                                 void* stream) {
+  cudaStream_t s = (cudaStream_t)stream;
+  BDE_REQUIRE(g != nullptr && dst != nullptr, "bde_shuffle2x_sum: null pointer");
+  BDE_REQUIRE(c > 0 && c % 8 == 0, "bde_shuffle2x_sum: c must be a positive multiple of 8 (got %d)", c);
+  BDE_REQUIRE(n_img >= 0 && h >= 0 && w >= 0, "bde_shuffle2x_sum: bad sizes");
+  BDE_REQUIRE(dtype == BDE_F32 || dtype == BDE_BF16, "bde_shuffle2x_sum: bad dtype %d", dtype);
+  BDE_REQUIRE(((uintptr_t)g | (uintptr_t)skip | (uintptr_t)dst) % 16 == 0, "bde_shuffle2x_sum: buffers must be 16-byte aligned");
+  const size_t rows = (size_t)n_img * 2 * h;
+  BDE_REQUIRE(rows < ((size_t)1 << 31) && (size_t)2 * w * c < ((size_t)1 << 31), "bde_shuffle2x_sum: map too large");
+  if (rows == 0 || w == 0) return 0;
+  const int esize = dtype == BDE_F32 ? 4 : 2;
+  const int cv = c * esize / 16;
+  const dim3 grid((unsigned)ceil_div((size_t)2 * w * cv, 256), (unsigned)(rows < 65535 ? rows : 65535));
+  if (dtype == BDE_F32)
+    shuffle2x_sum_kernel<float><<<grid, 256, 0, s>>>((const float*)g, (const float*)skip, h, w, cv, (int)rows, (float*)dst);
+  else
+    shuffle2x_sum_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>((const __nv_bfloat16*)g, (const __nv_bfloat16*)skip, h, w, cv,
+                                                             (int)rows, (__nv_bfloat16*)dst);
+  return check_launch("shuffle2x_sum_kernel");
 }
 
 extern "C" int bde_pred_sigmoid(const void* x, const void* head, const float* wt, const float* wt_head, const float* bias, int c,

@@ -7,11 +7,14 @@ Mirrors the reference interface:
 * ``UNetRecurrent(...)``: ``forward(x, prev_states) -> (img, states)`` -- model/e2vid/unet.py:139-200
 * ``state_dict`` keys ``unetrecurrent.{head,encoders.i.{conv,recurrent_block.Gates},resblocks.r.{conv1,conv2},
   decoders.i,pred}.*``                                    -- model/e2vid/submodules.py:16-44,78-128,212-306
+  (``decoders.i.transposed_conv2d.*`` with ``use_upsample_conv=False``: TransposedConvLayer, model/e2vid/submodules.py)
 
 One frame per call, batch is the parallel axis, recurrent state is carried between calls.  The modules are
 parameter containers; all arithmetic runs in libbde2vid_sm100.so (head / encoder / decoder convs, ConvLSTM gates
 conv with the pointwise update in its epilogue, ResidualBlock with the residual + ReLU in the second conv's
-epilogue, bilinear x2 of (skip + x) feeding the decoder conv, fused pred + sigmoid).  No CPU path exists.
+epilogue, bilinear x2 of (skip + x) feeding the decoder conv -- or, with ``use_upsample_conv=False``, the transposed
+decoder conv as one phase conv on the low-resolution map plus a pixel shuffle --, fused pred + sigmoid).  No CPU path
+exists.
 """
 import functools
 import os
@@ -21,7 +24,7 @@ import torch.nn as nn
 
 from . import ops
 from .engine import (VOX_CPAD, _Layer, _conv_layer, _f32, _fold_norm, _gru_layers, _lstm_layer, _pack_conv,
-                     _run_layer)
+                     _packed_conv, _run_layer)
 from .model import _ConvLayer, _RecurrentConv, _unsupported
 from .ops import ACT_NONE, ACT_RELU, ENGINE_SIMT, ENGINE_TCGEN05, EPI_GRU_OUT, EPI_GRU_UR, EPI_LSTM
 from .registry import MODELS
@@ -32,6 +35,33 @@ class _ResidualBlock(nn.Module):                  # model/e2vid/submodules.py:21
         super().__init__()
         self.conv1 = nn.Conv2d(c, c, 3, padding=1)
         self.conv2 = nn.Conv2d(c, c, 3, padding=1)
+
+
+class _TransposedConvLayer(nn.Module):            # model/e2vid/submodules.py TransposedConvLayer (norm=None, ReLU)
+    def __init__(self, cin, cout):
+        super().__init__()
+        self.transposed_conv2d = nn.ConvTranspose2d(cin, cout, 5, stride=2, padding=2, output_padding=1)
+
+
+def _transposed_layer(holder, dt, tc):
+    """Packs ``relu(ConvTranspose2d(Cin, Cout, 5, stride=2, padding=2, output_padding=1))`` as ONE 3x3, stride-1, pad-1
+    convolution over the low-resolution input with N = 4*Cout: output pixel (2i+py, 2j+px) only sees the input pixels
+    (i+dy, j+dx), |dy|, |dx| <= 1, through tap (py+2-2dy, px+2-2dx) of the 5x5 kernel, so phase p = 2py+px owns rows
+    [p*Cout, (p+1)*Cout) of W3[n, ci, dy+1, dx+1] (zero where the tap falls outside the kernel).  bde_shuffle2x_sum
+    moves phase p of pixel (i, j) to (2i+py, 2j+px); the ReLU commutes with that permutation and stays in the epilogue."""
+    ct = holder.transposed_conv2d
+    wt = ct.weight.detach().float()                             # [Cin, Cout, 5, 5] (ConvTranspose2d layout)
+    cin, cout, k, _ = wt.shape
+    w3 = wt.new_zeros(2, 2, cout, cin, 3, 3)
+    for py in range(2):
+        for px in range(2):
+            for dy in (-1, 0, 1):
+                for dx in (-1, 0, 1):
+                    ky, kx = py + 2 - 2 * dy, px + 2 - 2 * dx
+                    if ky < k and kx < k:
+                        w3[py, px, :, :, dy + 1, dx + 1] = wt[:, :, ky, kx].t()
+    b4 = ct.bias.detach().float().repeat(4)
+    return _packed_conv(w3.reshape(4 * cout, cin, 3, 3), b4, 1, dt, tc, cin % 64 == 0)
 
 
 class LSTMState:
@@ -85,19 +115,21 @@ class UNetRecurrent(nn.Module):
             norm = None
         if norm is not None:
             _unsupported("norm=%r in the E2VID family (ResidualBlock bn1 / bn2, model/e2vid/submodules.py:212-247)" % (norm,))
-        if not use_upsample_conv:
-            _unsupported("TransposedConvLayer decoders")
         if num_bins > VOX_CPAD:
             _unsupported("num_bins > %d" % VOX_CPAD)
         self.num_bins, self.num_encoders = num_bins, num_encoders
         self.base_num_channels, self.num_residual_blocks = base_num_channels, num_residual_blocks
         bc, ne = base_num_channels, num_encoders
         self.recurrent_block_type = recurrent_block_type
+        self.use_upsample_conv = use_upsample_conv
         self.head = _ConvLayer(num_bins, bc, 5)
         self.encoders = nn.ModuleList([_RecurrentConv(bc * 2 ** i, bc * 2 ** (i + 1), 5, norm, recurrent_block_type)
                                        for i in range(ne)])
         self.resblocks = nn.ModuleList([_ResidualBlock(bc * 2 ** ne) for _ in range(num_residual_blocks)])
-        self.decoders = nn.ModuleList([_ConvLayer(bc * 2 ** (ne - i), bc * 2 ** (ne - i - 1), 5, norm) for i in range(ne)])
+        if use_upsample_conv:     # UpsampleConvLayer (unet.py self.UpsampleLayer)
+            self.decoders = nn.ModuleList([_ConvLayer(bc * 2 ** (ne - i), bc * 2 ** (ne - i - 1), 5, norm) for i in range(ne)])
+        else:                     # TransposedConvLayer
+            self.decoders = nn.ModuleList([_TransposedConvLayer(bc * 2 ** (ne - i), bc * 2 ** (ne - i - 1)) for i in range(ne)])
         self.pred = _ConvLayer(bc, num_output_channels, 1)
         self.precision = os.environ.get("BDE2VID_PRECISION", "bf16")
         self._packed = None
@@ -133,7 +165,8 @@ class UNetRecurrent(nn.Module):
                       if self.recurrent_block_type == 'convlstm' else _gru_layers(e.recurrent_block, dt, tc))
                      for e in self.encoders],
                 res=[(_conv_layer(r.conv1, 1, dt, tc), _conv_layer(r.conv2, 1, dt, tc)) for r in self.resblocks],
-                dec=[_conv_layer(d, 1, dt, tc) for d in self.decoders],
+                dec=[_conv_layer(d, 1, dt, tc) if self.use_upsample_conv else _transposed_layer(d, dt, tc)
+                     for d in self.decoders],
                 pred_w=_f32(self.pred.conv2d.weight.reshape(-1)), pred_b=_f32(self.pred.conv2d.bias))
             hw, hb = _fold_norm(self.head.conv2d, self.head)
             # dedicated first-layer kernel (planar fp32 voxels -> NHWC bf16): 32 channels, 5x5, as in the BDE2VID engine
@@ -156,7 +189,13 @@ class UNetRecurrent(nn.Module):
         b["res"] = [E(B, lv["h"], lv["w"], lv["C"]) for _ in range(3)]
         for i in range(ne):
             lv = b["lv"][ne - 1 - i]
-            b["dec"].append(dict(up=E(B, 2 * lv["h"], 2 * lv["w"], lv["C"]), out=E(B, 2 * lv["h"], 2 * lv["w"], lv["C"] // 2)))
+            if self.use_upsample_conv:
+                b["dec"].append(dict(up=E(B, 2 * lv["h"], 2 * lv["w"], lv["C"]), out=E(B, 2 * lv["h"], 2 * lv["w"], lv["C"] // 2)))
+            else:
+                # g: the four phase outputs [.., 4 * Cout] of the low-resolution conv; out: shuffled (+ next skip)
+                b["dec"].append(dict(g=E(B, lv["h"], lv["w"], 2 * lv["C"]), out=E(B, 2 * lv["h"], 2 * lv["w"], lv["C"] // 2)))
+        if not self.use_upsample_conv:
+            b["sum0"] = E(B, b["lv"][-1]["h"], b["lv"][-1]["w"], b["lv"][-1]["C"])    # decoder 0 input x + blocks[ne-1]
         self._bufs = {key: b}
         return b
 
@@ -224,14 +263,27 @@ class UNetRecurrent(nn.Module):
             dst = r[j & 1]
             G(c2l, r[2], dst, B, ch, cw, cc, act=ACT_RELU, residual=cur, res_mode=1)
             cur = dst
-        # decoders: UpsampleConvLayer(skip_sum(x, block))   (unet.py:193-195; ReLU, e2vid/submodules.py:78-106)
-        for i in range(ne):
-            lv = bufs["lv"][ne - 1 - i]
-            dd = bufs["dec"][i]
-            blk = states[ne - 1 - i].h_nhwc
-            ops.upsample2x_sum(blk, cur, 1.0, B, lv["h"], lv["w"], lv["C"], dd["up"])
-            G(P["dec"][i], dd["up"], dd["out"], B, 2 * lv["h"], 2 * lv["w"], lv["C"], act=ACT_RELU)
-            cur = dd["out"]
+        if self.use_upsample_conv:
+            # decoders: UpsampleConvLayer(skip_sum(x, block))   (unet.py:193-195; ReLU, e2vid/submodules.py:78-106)
+            for i in range(ne):
+                lv = bufs["lv"][ne - 1 - i]
+                dd = bufs["dec"][i]
+                blk = states[ne - 1 - i].h_nhwc
+                ops.upsample2x_sum(blk, cur, 1.0, B, lv["h"], lv["w"], lv["C"], dd["up"])
+                G(P["dec"][i], dd["up"], dd["out"], B, 2 * lv["h"], 2 * lv["w"], lv["C"], act=ACT_RELU)
+                cur = dd["out"]
+        else:
+            # decoders: TransposedConvLayer(skip_sum(x, block)) as the phase conv on the low-resolution map, then the
+            # shuffle to 2h x 2w, which also adds the NEXT decoder's skip (the last decoder's output has none)
+            ops.add(cur, states[ne - 1].h_nhwc, out_t=bufs["sum0"], dtype=dt)
+            cur = bufs["sum0"]
+            for i in range(ne):
+                lv = bufs["lv"][ne - 1 - i]
+                dd = bufs["dec"][i]
+                G(P["dec"][i], cur, dd["g"], B, lv["h"], lv["w"], lv["C"], act=ACT_RELU)
+                skip = states[ne - 2 - i].h_nhwc if i < ne - 1 else None
+                ops.shuffle2x_sum(dd["g"], skip, B, lv["h"], lv["w"], lv["C"] // 2, dd["out"])
+                cur = dd["out"]
         ops.pred_sigmoid(cur, bufs["head"], P["pred_w"], P["pred_b"], bc, B * H * W, bufs["img"])
         return bufs["img"].clone().view(B, 1, H, W), states
 

@@ -180,6 +180,15 @@ def upsample2x_sum(skip, x, x_scale, n_img, h, w, c, dst):
     return dst
 
 
+def shuffle2x_sum(g, skip, n_img, h, w, c, dst):
+    """dst [n_img, 2h, 2w, c] = phase shuffle of g [n_img, h, w, 4c] (+ skip, same shape as dst); see bde_shuffle2x_sum."""
+    lib = _lib.require_device()
+    assert g.dtype == dst.dtype and (skip is None or skip.dtype == dst.dtype), "g, skip and dst must share one dtype"
+    check(lib.bde_shuffle2x_sum(ptr(g), ptr(skip), n_img, h, w, c, ptr(dst), BDE_DTYPE[dst.dtype], stream_ptr()),
+          "bde_shuffle2x_sum")
+    return dst
+
+
 def pred_sigmoid(x, head, wt, bias, c, n_pix, img, wt_head=None, act=ACT_SIGMOID):
     lib = _lib.require_device()
     check(lib.bde_pred_sigmoid(ptr(x), ptr(head), ptr(wt), ptr(wt_head), ptr(bias), c, n_pix, ptr(img), BDE_DTYPE[x.dtype],

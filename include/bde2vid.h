@@ -230,6 +230,15 @@ int bde_add(const void* a, int a_f32, const void* b, int b_f32, float* out_f32, 
 int bde_upsample2x_sum(const void* skip, int skip_f32, const void* x, int x_f32, float x_scale,
                        int n_img, int h, int w, int c, void* dst, int dtype, void* stream);
 
+/* Pixel shuffle of a stride-2 transposed convolution computed as four stride-1 phase convolutions on the
+ * low-resolution map (TransposedConvLayer of model/e2vid/submodules.py, E2VID's use_upsample_conv=False), plus the
+ * skip_sum that feeds the next decoder (model/e2vid/unet.py):
+ *   dst[b, 2i+py, 2j+px, :] = g[b, i, j, (2py+px)*c : (2py+px+1)*c]  (+ skip[b, 2i+py, 2j+px, :])
+ * g NHWC [n_img, h, w, 4c]; skip (NULL = none) and dst NHWC [n_img, 2h, 2w, c]; all three of `dtype`, 16-byte
+ * aligned; c % 8 == 0.  A bf16 sum is formed in fp32 and rounded once. */
+int bde_shuffle2x_sum(const void* g, const void* skip, int n_img, int h, int w, int c, void* dst, int dtype,
+                      void* stream);
+
 /* img[p] = act(bias + sum_c wt[c] * x[p,c] + wt_head[c] * head[p,c])  (predI + output activation, ...V5.py:195-197)
  * x, head NHWC [P, c] of `dtype`; img float32[P].  wt_head = NULL means wt (skip_type 'sum': w . (x + head)); with
  * skip_type 'concat' the two 1x1 convolutions of predI (...V5.py:92-97: fusion 2c -> c, then c -> 1, no activation in
